@@ -5,6 +5,7 @@
                     [--batch 32] [--seconds 4] [--engine auto|generic|tensor]
                     [--total-utterances 1024 --micro-batch 16]   (cfg-3: strong scaling of a fixed job over the ranks)
                     [--loss]                                     (cfg-5: forward + PIT SI-SNR loss, data-parallel mean)
+                    [--dump-outputs DIR]                         (what the last timed step computed, as DIR/<name>.npy)
 
 One "step" = one forward pass of DPTN-AV (src/configs/model/dptn_wav_av.yaml) over one batch of
 synthetic 16 kHz mixtures + synthetic lip embeddings, followed by the PIT SI-SNRi reduction.
@@ -44,6 +45,7 @@ OTHER_MODELS = {
 }
 METRIC = "dptn_av_separated_audio_seconds_per_second"
 UNIT = "audio-s/s"
+DUMP_LIMIT = 64 << 20    # bytes --dump-outputs writes at most, .npy headers included
 
 
 def geometry(T):
@@ -121,6 +123,27 @@ def make_batch(B, T, seed):
     e1 = torch.randn(B, 512, Tv, generator=g)
     e2 = torch.randn(B, 512, Tv, generator=g)
     return s1 + s2, s1, s2, e1, e2
+
+
+def dump_outputs(arrays, out_dir):
+    """Writes every tensor of `arrays` as out_dir/<name>.npy (float32, or float64 where the path computes in float64) so
+    that two builds can be compared output for output.  Arrays of up to 1 MiB are written whole; above DUMP_LIMIT in all,
+    each larger array is cut to the same fraction of its flattened elements, a fixed, seeded sample in ascending index
+    order, identical from run to run."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+    arrays = {k: a if a.dtype in (np.float32, np.float64) else a.astype(np.float32) for k, a in arrays.items()}
+    large = {k for k, a in arrays.items() if a.nbytes > (1 << 20)}
+    # 256 bytes bound one .npy header
+    budget = DUMP_LIMIT - 256 * len(arrays) - sum(a.nbytes for k, a in arrays.items() if k not in large)
+    total = sum(arrays[k].nbytes for k in large)
+    for name, a in arrays.items():
+        if name in large and total > budget:
+            n = a.size * budget // total
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, n, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 class ClockSampler:
@@ -221,7 +244,14 @@ def main():
                     help="cfg-3: a fixed job of this many utterances, sharded over the ranks (strong scaling)")
     ap.add_argument("--micro-batch", type=int, default=32)
     ap.add_argument("--loss", action="store_true", help="cfg-5: every step also computes the PIT SI-SNR loss")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (separated waveforms, SI-SNR rows and summary, loss) as DIR/<name>.npy; "
+                         "the inputs are seeded, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -335,14 +365,21 @@ def main():
             loss = loss / world
         return loss
 
+    last = {}    # what the latest step computed, for --dump-outputs
+
     def step_resident():
         out = fwd(mix, e1, e2)
-        rows, rows_loss, _ = V.pit_sisnr_all(out["s1_pred"], out["s2_pred"], s1, s2, mix)
+        rows, rows_loss, summary = V.pit_sisnr_all(out["s1_pred"], out["s2_pred"], s1, s2, mix)
+        last.update(s1_pred=out["s1_pred"], s2_pred=out["s2_pred"], sisnr_rows=rows, sisnr_loss_rows=rows_loss,
+                    sisnr_summary=summary)
         if args.loss:
-            step_loss(out)
+            last["loss"] = step_loss(out)
         # N > 1: the NCCL all-reduce of the SI-SNR sums is issued every step, stream-ordered; the reduced vector stays on
         # the device (an evaluation loop reads it once per partition, not once per batch)
-        return all_reduce_sisnr_sums(sisnr_sums(rows, rows_loss)) if world > 1 else rows
+        if world > 1:
+            last["sisnr_sums"] = all_reduce_sisnr_sums(sisnr_sums(rows, rows_loss))
+            return last["sisnr_sums"]
+        return rows
 
     # End-to-end step through the public nn.Module / metric API from PINNED HOST buffers.  Input copies are double
     # buffered the way an evaluation loop over a DataLoader runs (speech_separation_b200.Inferencer): while step k
@@ -410,6 +447,8 @@ def main():
     total_ms, wall = timed(step_resident, args.steps)
     launches = lib.vatss_launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else {}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last, args.dump_outputs)
 
     for _ in range(2):
         step_e2e()

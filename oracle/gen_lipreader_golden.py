@@ -8,6 +8,7 @@ synthetic weights of oracle.lipreader_oracle.make_state_dict (strict=False: the 
 init and is not on the path), runs the reference preprocessing classes (Normalize, CenterCrop, Normalize -
 dataloaders.py:24-27; `cv2`, which preprocess.py imports for an unrelated transform, is not installed and is stubbed
 by an empty module) and the reference forward, and stores the raw frames (uint8) and the (B, T, 512) features.
+`python -m oracle.gen_lipreader_golden preprocess` writes tests/golden/lipreader_preprocess.npz (write_preprocess_golden).
 """
 import importlib
 import json
@@ -22,6 +23,8 @@ from . import lipreader_oracle as LO
 
 REF_ROOT = os.environ.get("VATSS_REFERENCE_ROOT", "/root/reference")
 OUT_DIR = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
+# square, non-square and odd frame sizes: the crop offsets round half the excess
+PREPROCESS_SIZES = ((96, 96), (88, 88), (97, 101), (120, 90), (89, 96))
 
 
 def load_reference():
@@ -54,7 +57,7 @@ def build_reference(model_mod, relu_type):
 
 def main():
     model_mod, pre = load_reference()
-    pipeline = pre.Compose([pre.Normalize(0.0, 255.0), pre.CenterCrop((88, 88)), pre.Normalize(0.421, 0.165)])
+    pipeline = reference_pipeline(pre)
     for relu_type, (B, T) in (("swish", (2, 7)), ("prelu", (1, 5)), ("relu", (1, 5))):
         torch.manual_seed(0)
         ref = build_reference(model_mod, relu_type).eval()
@@ -76,5 +79,32 @@ def main():
         print(path, feats.shape, float(np.abs(feats).mean()), os.path.getsize(path))
 
 
+def reference_pipeline(pre):
+    """dataloaders.py:24-27 built from the reference's own preprocessing classes."""
+    return pre.Compose([pre.Normalize(0.0, 255.0), pre.CenterCrop((88, 88)), pre.Normalize(0.421, 0.165)])
+
+
+def write_preprocess_golden():
+    """tests/golden/lipreader_preprocess.npz: 3 frames per size of PREPROCESS_SIZES (default_rng(1)) and what
+    Normalize(0, 255) -> CenterCrop(88, 88) -> Normalize(0.421, 0.165) makes of them.  Computed by the reference's classes
+    where its checkout is present, otherwise by the restatement LO.preprocess; `source` records which."""
+    if os.path.isfile(os.path.join(REF_ROOT, "src", "lipreader", "lipreading", "preprocess.py")):
+        pipeline, source = reference_pipeline(load_reference()[1]), "reference preprocess.py classes"
+    else:
+        pipeline, source = LO.preprocess, "oracle.lipreader_oracle.preprocess (reference checkout not present)"
+    rng = np.random.default_rng(1)
+    out = {"sizes": np.array(PREPROCESS_SIZES, dtype=np.int64), "source": np.array(source)}
+    for i, (h, w) in enumerate(PREPROCESS_SIZES):
+        frames = rng.integers(0, 256, (3, h, w)).astype(np.float32)
+        out[f"c{i}.frames"] = frames.astype(np.uint8)
+        out[f"c{i}.want"] = np.asarray(pipeline(frames), dtype=np.float32)
+    path = os.path.join(OUT_DIR, "lipreader_preprocess.npz")
+    np.savez_compressed(path, **out)
+    print(path, source, os.path.getsize(path))
+
+
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] == ["preprocess"]:
+        write_preprocess_golden()
+    else:
+        main()

@@ -301,22 +301,28 @@ def test_make_embeddings_end_to_end_on_the_device(golden_dir, tmp_path):
         assert rel_l2(e.T, feats[b]) < TENSOR_TOL
 
 
-def test_preprocessing_matches_reference_classes_when_available():
-    """`center_crop_window` / `LO.preprocess` against the reference's own CenterCrop / Normalize classes for several frame
-    sizes (only where /root/reference exists: the build container; the committed goldens cover the 96 x 96 case anywhere)."""
+def test_preprocessing_matches_reference_classes_when_available(golden_dir):
+    """`center_crop_window` / `LO.preprocess` for square, non-square and odd frame sizes against the stored output of the
+    Normalize / CenterCrop / Normalize pipeline (tests/golden/lipreader_preprocess.npz, oracle/gen_lipreader_golden.py),
+    and, where a checkout of the reference is present, against the reference's own classes as well."""
     from oracle import ref_import
-
-    if not ref_import.available():
-        pytest.skip("reference checkout not present")
-    from oracle.gen_lipreader_golden import load_reference
+    from oracle.gen_lipreader_golden import PREPROCESS_SIZES
     from speech_separation_b200.lipreader import center_crop_window
 
-    _, pre = load_reference()
-    pipeline = pre.Compose([pre.Normalize(0.0, 255.0), pre.CenterCrop((88, 88)), pre.Normalize(0.421, 0.165)])
+    z = np.load(os.path.join(golden_dir, "lipreader_preprocess.npz"))
+    assert [tuple(s) for s in z["sizes"]] == list(PREPROCESS_SIZES)
+    pipeline = None
+    if ref_import.available():
+        from oracle.gen_lipreader_golden import load_reference, reference_pipeline
+
+        pipeline = reference_pipeline(load_reference()[1])
     rng = np.random.default_rng(1)
-    for h, w in ((96, 96), (88, 88), (97, 101), (120, 90), (89, 96)):
+    for i, (h, w) in enumerate(PREPROCESS_SIZES):
         frames = rng.integers(0, 256, (3, h, w)).astype(np.float32)
-        want = pipeline(frames)
+        assert np.array_equal(frames, z[f"c{i}.frames"])
+        want = z[f"c{i}.want"]
+        if pipeline is not None:
+            np.testing.assert_allclose(pipeline(frames), want, rtol=1e-6, atol=1e-6)
         y0, x0, th, tw = center_crop_window(h, w)
         assert want.shape == (3, th, tw)
         got = (frames[:, y0:y0 + th, x0:x0 + tw] / 255.0 - 0.421) / 0.165
