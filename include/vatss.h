@@ -210,6 +210,15 @@ int vatss_tc_lstm(const void* x16, const void* x16lo /* NULL, or half(x - half(x
 int vatss_tc_attention(const void* qkv16, void* out16, int mode, int B, int S, int C, int N, int heads, int force_simt,
                        void* stream);
 
+/* vatss_tc_tail: the TENSOR engine's separator tail on its own - speaker split, overlap-add with the centred pad,
+ * post-conv (or masking) head and decoder - through the same dispatch vatss_forward runs after its last block.
+ * x16 (B,S,C,N) fp16 token-major = PReLU(x) as the last block's epilogue writes it; enc (B,L,N) f32;
+ * d / params / packed as for vatss_forward (d must select the TENSOR engine); s1_pred, s2_pred (B,T) f32;
+ * workspace >= vatss_workspace_bytes(d, B, T, 0). */
+int vatss_tc_tail(const vatss_model_desc* d, const float* const* params, int n_params, const void* packed,
+                  const void* x16, const float* enc, int B, int T, float* s1_pred, float* s2_pred,
+                  void* workspace, size_t workspace_bytes, void* stream);
+
 /* Instrumentation (no reference counterpart; used by bench.py).
  * vatss_launch_count: number of kernels this library has launched in this process.
  * vatss_profile_begin: start recording CUDA-event pairs around the stages of subsequent calls

@@ -118,10 +118,12 @@ def interp_linear_index(L, Tv, dtype=np.float64):
     return i0, i1, lam
 
 
-def av_fuse(enc, emb1, emb2, P):
+def av_fuse(enc, emb1, emb2, P, index=None):
     """F1: tanh-gated lip-embedding fusion (dptn_wav.py:173-184).
 
     enc (B,L,N) token-major; emb* (B,E,Tv).  compress -> concat -> interpolate -> LN -> gate.
+    index: the interpolation's (i0, i1, lam), default interp_linear_index(L, Tv, enc.dtype); tests pass the float32
+    source indices of a float32 implementation to compare everything else in enc.dtype.
     """
     Wv, bv = P["visual_compression.weight"], P["visual_compression.bias"]
     v1 = np.einsum("bet,je->btj", emb1, Wv) + bv
@@ -129,7 +131,7 @@ def av_fuse(enc, emb1, emb2, P):
     v = np.concatenate([v1, v2], axis=-1)  # (B,Tv,N)
     L = enc.shape[1]
     Tv = v.shape[1]
-    i0, i1, lam = interp_linear_index(L, Tv, dtype=enc.dtype)
+    i0, i1, lam = interp_linear_index(L, Tv, dtype=enc.dtype) if index is None else index
     vi = (1.0 - lam)[None, :, None] * v[:, i0, :] + lam[None, :, None] * v[:, i1, :]
     g = np.tanh(P["gate"][0])
     return enc + g * layer_norm(vi, P["video_ln.weight"], P["video_ln.bias"])
@@ -281,11 +283,12 @@ def dual_path_blocks(x, P, cfg: PathConfig, taps=None):
     return x
 
 
-def separator_tail(x, enc, P, cfg: PathConfig, taps=None):
+def separator_tail(x, enc, P, cfg: PathConfig, taps=None, round_ola=None):
     """T1+S3: PReLU -> 1x1 Conv2d(N->2N) -> overlap-add -> centred pad -> speaker split -> head.
 
     dptn_wav.py:47-59 (dptn.py:129-141 for the masking variant, dprnn.py:213-225).
     x (B,S,C,N) token-major, enc (B,L,N).  Returns the two decoder inputs u_j (B,L,N).
+    round_ola: optional map applied to the overlap-added tensor (tests: the fp16 rounding an engine stores it with).
     """
     B, S, C, N = x.shape
     L = enc.shape[1]
@@ -299,6 +302,8 @@ def separator_tail(x, enc, P, cfg: PathConfig, taps=None):
         ola[:, Pstep * s : Pstep * s + C, :] += y[:, s, :, :]
     d = L - ola.shape[1]
     ola = np.pad(ola, [(0, 0), (d // 2, d - d // 2), (0, 0)])
+    if round_ola is not None:
+        ola = round_ola(ola)
     if taps is not None:
         taps["ola"] = ola
     outs = []

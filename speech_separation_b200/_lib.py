@@ -73,6 +73,10 @@ EXPORTS = {
     "vatss_tc_lstm": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.POINTER(ctypes.c_void_p), ctypes.c_void_p] +
                       [ctypes.c_int] * 7 + [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
     "vatss_tc_attention": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p] + [ctypes.c_int] * 7 + [ctypes.c_void_p]),
+    "vatss_tc_tail": (ctypes.c_int, [ctypes.POINTER(ModelDesc), ctypes.POINTER(ctypes.c_void_p), ctypes.c_int,
+                                     ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int,
+                                     ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t,
+                                     ctypes.c_void_p]),
     "vatss_launch_count": (ctypes.c_ulonglong, []),
     "vatss_engine_fallback_reason": (ctypes.c_char_p, [ctypes.POINTER(ModelDesc)]),
     "vatss_debug_lstm_trace": (None, [ctypes.c_void_p]),

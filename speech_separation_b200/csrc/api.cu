@@ -427,6 +427,22 @@ int vatss_tc_attention(const void* qkv16, void* out16, int mode, int B, int S, i
                               (cudaStream_t)stream);
 }
 
+int vatss_tc_tail(const vatss_model_desc* d, const float* const* params, int n_params, const void* packed,
+                  const void* x16, const float* enc, int B, int T, float* s1_pred, float* s2_pred, void* workspace,
+                  size_t workspace_bytes, void* stream) {
+  if (check_desc(d)) return -1;
+  VATSS_CHECK_ARG(params != nullptr && n_params == n_params_of(d), "parameter table has %d entries, expected %d",
+                  n_params, n_params_of(d));
+  VATSS_CHECK_ARG(tensor_engine_selected(d), "tc_tail: the model does not run on the TENSOR engine");
+  VATSS_CHECK_ARG(packed && x16 && enc && s1_pred && s2_pred && workspace, "tc_tail: NULL pointer");
+  Geometry g;
+  if (geometry(d, B, T, 0, &g)) return -1;
+  const size_t need = vatss_workspace_bytes(d, B, T, 0);
+  VATSS_CHECK_ARG(workspace_bytes >= need, "workspace too small: %zu bytes given, %zu needed", workspace_bytes, need);
+  return tensor_engine_tail(d, params, packed, (const __half*)x16, enc, g.B, g.T, 0, g.L, g.S, s1_pred, s2_pred,
+                            workspace, (cudaStream_t)stream);
+}
+
 void vatss_debug_lstm_trace(void* dev_buffer) { vatss::g_lstm_trace = (long long*)dev_buffer; }
 void vatss_debug_cta_limit(int ctas) { vatss::g_cta_limit = ctas; }
 void vatss_debug_lstm_pingpong(int on) { vatss::g_lstm_pingpong = on; }

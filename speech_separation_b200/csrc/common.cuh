@@ -144,8 +144,6 @@ int launch_fold_spk(const float* wfold, const float* Wspk, const float* bspk, in
                     cudaStream_t st);
 int launch_tail_fused(const __half* px, const float* enc, const float* w2, const float* c2, const float* wdT,
                       const float* cfold, int B, int S, int C, int P, int L, int N, int K, float* proj, cudaStream_t st);
-int launch_ola_decode(const float* y, const float* enc, const float* wfold, const float* wdT, const float* cfold, int B,
-                      int S, int C, int P, int L, int N, int K, float* proj, cudaStream_t st);
 
 // sisnr.cu
 int sisnr_chunks(int T);

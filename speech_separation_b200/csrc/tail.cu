@@ -61,9 +61,8 @@ int launch_ola_token_major(const float* y, int B, int S, int C, int P, int L, in
 // split and the decoder's overlap-add is linear per frame,
 //   frames[b,l,spk,k] = sum_n Wd[n,k] (sum_m Whead[n,m] ola[b,l,spk*N+m] + bhead[n] + enc[b,l,n])
 //                     = sum_m wfold[k,m] ola[...] + sum_n Wd[n,k] enc[b,l,n] + cfold[k],
-// with wfold = Wd^T Whead and cfold = Wd^T bhead folded at weight-pack time.  One warp per frame gathers the
-// <= 2 overlapping chunk rows of the speaker-split output (fp32), adds them and applies both K x N projections:
-// the overlap-added tensor, the head output and their fp16 copies (2.4 GB of traffic) never exist.
+// with wfold = Wd^T Whead and cfold = Wd^T bhead folded at weight-pack time (k_tail_fused below folds the speaker
+// split in as well): the overlap-added tensor, the head output and their fp16 copies (2.4 GB of traffic) never exist.
 // ----------------------------------------------------------------------------------------
 __global__ void k_fold_head(const float* __restrict__ Whead, const float* __restrict__ bhead,
                             const float* __restrict__ Wd, int N, int K, float* __restrict__ wfold,
@@ -88,76 +87,6 @@ int launch_fold_head(const float* Whead, const float* bhead, const float* Wd, in
   k_fold_head<<<(K * N + 127) / 128, 128, 0, st>>>(Whead, bhead, Wd, N, K, wfold, wdT, cfold);
   VATSS_LAUNCH_OK();
   return 0;
-}
-
-template <int N, int K>
-__global__ void __launch_bounds__(128)
-k_ola_decode(const float* __restrict__ y, const float* __restrict__ enc, const float* __restrict__ wfold,
-             const float* __restrict__ wdT, const float* __restrict__ cfold, int S, int C, int P, int L, int padl,
-             int Lo, long long frames, float* __restrict__ proj) {
-  constexpr int CPL = N / 16;   // channels per lane: lanes 0-15 take speaker 0, lanes 16-31 speaker 1
-  const int lane = threadIdx.x & 31, h = lane >> 4, j = lane & 15;
-  // this lane's slice of both projections lives in registers for the whole grid-stride loop (measured: reading
-  // them from shared memory instead, with twice the resident warps, is 20 % slower)
-  float wf[K][CPL], wd[K][CPL], ck[K];
-#pragma unroll
-  for (int k = 0; k < K; ++k) {
-    ck[k] = cfold[k];
-#pragma unroll
-    for (int i = 0; i < CPL; ++i) {
-      wf[k][i] = wfold[k * N + j * CPL + i];
-      wd[k][i] = wdT[k * N + j * CPL + i];
-    }
-  }
-  const long long warp0 = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  const long long nwarps = (long long)gridDim.x * (blockDim.x >> 5);
-  for (long long row = warp0; row < frames; row += nwarps) {
-    const int b = (int)(row / L);
-    const int t = (int)(row - (long long)b * L) - padl;
-    float o[CPL], e[CPL];
-#pragma unroll
-    for (int i = 0; i < CPL; ++i) o[i] = 0.f;
-    {
-      const float4* ep = reinterpret_cast<const float4*>(enc + row * N + j * CPL);
-#pragma unroll
-      for (int i = 0; i < CPL / 4; ++i) {
-        const float4 v = ep[i];
-        e[4 * i] = v.x; e[4 * i + 1] = v.y; e[4 * i + 2] = v.z; e[4 * i + 3] = v.w;
-      }
-    }
-    if (t >= 0 && t < Lo) {
-      int s_lo = t - C + 1 + P - 1;
-      s_lo = s_lo <= 0 ? 0 : s_lo / P;
-      int s_hi = t / P;
-      if (s_hi > S - 1) s_hi = S - 1;
-      for (int s = s_lo; s <= s_hi; ++s) {
-        const float4* yp =
-            reinterpret_cast<const float4*>(y + (((long long)b * S + s) * C + (t - P * s)) * (2 * N) + h * N + j * CPL);
-#pragma unroll
-        for (int i = 0; i < CPL / 4; ++i) {
-          const float4 v = yp[i];
-          o[4 * i] += v.x; o[4 * i + 1] += v.y; o[4 * i + 2] += v.z; o[4 * i + 3] += v.w;
-        }
-      }
-    }
-    float acc[K];
-#pragma unroll
-    for (int k = 0; k < K; ++k) {
-      float a = 0.f;
-#pragma unroll
-      for (int i = 0; i < CPL; ++i) a = fmaf(wf[k][i], o[i], fmaf(wd[k][i], e[i], a));
-      // sum over the 16 lanes of this speaker's half-warp
-      a += __shfl_xor_sync(0xffffffffu, a, 8);
-      a += __shfl_xor_sync(0xffffffffu, a, 4);
-      a += __shfl_xor_sync(0xffffffffu, a, 2);
-      a += __shfl_xor_sync(0xffffffffu, a, 1);
-      acc[k] = a + ck[k];
-    }
-    if (j == 0) {
-#pragma unroll
-      for (int k = 0; k < K; ++k) proj[(row * 2 + h) * K + k] = acc[k];
-    }
-  }
 }
 
 // ----------------------------------------------------------------------------------------
@@ -244,11 +173,16 @@ k_tail_fused(const __half* __restrict__ px, const float* __restrict__ enc, const
           const float2 v = __ldg(reinterpret_cast<const float2*>(enc + row * N + n0));
           e[f][0] = v.x; e[f][1] = v.y;
         }
+        int s_lo = 0, s_hi = -1;
         if (t >= 0 && t < Lo) {
-          int s_lo = t - C + 1 + P - 1;
+          s_lo = t - C + 1 + P - 1;
           s_lo = s_lo <= 0 ? 0 : s_lo / P;
-          int s_hi = t / P;
+          s_hi = t / P;
           if (s_hi > S - 1) s_hi = S - 1;
+        }
+        // s_lo > s_hi: a frame of the centred pad, or (step_size > chunk_size) a frame between two chunks that no
+        // chunk covers - the reference's fold leaves it at zero, so nothing is loaded and no split bias is added
+        if (s_lo <= s_hi) {
           nrows[f] = s_hi - s_lo + 1;
           // two rows for the 50 % overlap of the reference configs: both loads are issued unconditionally (the second
           // one re-reads the first row when there is only one) so that nothing depends on a data-dependent loop
@@ -552,28 +486,6 @@ int launch_tail_fused(const __half* px, const float* enc, const float* w2, const
   VATSS_TAIL_FUSED(64, 2)
   VATSS_TAIL_FUSED(128, 2)
 #undef VATSS_TAIL_FUSED
-  return 1;
-}
-
-// returns 1 when the (N, K) pair has no fused instance (caller falls back to the unfused sequence)
-int launch_ola_decode(const float* y, const float* enc, const float* wfold, const float* wdT, const float* cfold, int B,
-                      int S, int C, int P, int L, int N, int K, float* proj, cudaStream_t st) {
-  const long long frames = (long long)B * L;
-  if (frames == 0) return 0;
-  const int Lo = (S - 1) * P + C;
-  const int padl = (L - Lo) / 2;
-  const int blocks = (int)(ceil_div(frames, 4) < 148 * 12 ? ceil_div(frames, 4) : 148 * 12);
-#define VATSS_OLA_DECODE(NN, KK)                                                                                   \
-  if (N == NN && K == KK) {                                                                                        \
-    k_ola_decode<NN, KK><<<blocks, 128, 0, st>>>(y, enc, wfold, wdT, cfold, S, C, P, L, padl, Lo, frames, proj);   \
-    VATSS_LAUNCH_OK();                                                                                             \
-    return 0;                                                                                                      \
-  }
-  VATSS_OLA_DECODE(128, 7)
-  VATSS_OLA_DECODE(64, 7)
-  VATSS_OLA_DECODE(64, 2)
-  VATSS_OLA_DECODE(128, 2)
-#undef VATSS_OLA_DECODE
   return 1;
 }
 

@@ -170,6 +170,7 @@ const char* tensor_engine_unsupported_reason(const vatss_model_desc* d) {
     const int hd = d->N / d->heads;
     if (d->N % d->heads != 0 || (hd != 16 && hd != 32)) return "attention head dim not in {16, 32}";
   }
+  if (d->num_blocks == 0) return "no dual-path blocks (the tail reads PReLU(x) from the last block's epilogue)";
   if (d->num_blocks > 32) return "more than 32 dual-path blocks";
   return nullptr;
 }
@@ -235,7 +236,7 @@ int tensor_engine_forward(const vatss_model_desc* d, const float* const* params,
   Work w;
   carve_work(d, B, Tv, L, S, workspace, &w);
   const int N = d->N, H = d->H, C = d->C;
-  const long long tok = (long long)B * S * C, fr = (long long)B * L;
+  const long long tok = (long long)B * S * C;
   const bool dprnn = d->kind == VATSS_KIND_DPRNN, av = d->kind == VATSS_KIND_DPTN_AV;
   // DPTN residual stream.  Default: fp32 between sub-blocks, the LayerNorm-1 output y only as fp16 (it is the LSTM
   // operand anyway and re-enters as the FFN residual).  F16RES: the block residual is fp16 as well (1e-3 budget:
@@ -311,16 +312,26 @@ int tensor_engine_forward(const vatss_model_desc* d, const float* const* params,
           return rc;
       }
     }
-  // tail: (PReLU already applied to the fp16 copy) speaker split -> overlap-add -> head -> decoder
+  // the last block's epilogue left PReLU(x) in the fp16 copy
+  return tensor_engine_tail(d, params, packed, w.xa16, w.enc32, B, T, Tv, L, S, s1_pred, s2_pred, workspace, st);
+}
+
+// tail: speaker split -> overlap-add -> head -> decoder, on x16 = PReLU(x) (fp16, token-major) and the encoder output
+int tensor_engine_tail(const vatss_model_desc* d, const float* const* params, const void* packed, const __half* x16,
+                       const float* enc32, int B, int T, int Tv, int L, int S, float* s1_pred, float* s2_pred,
+                       void* workspace, cudaStream_t st) {
+  Packed p;
+  carve_packed(d, const_cast<void*>(packed), &p);
+  Work w;
+  carve_work(d, B, Tv, L, S, workspace, &w);
+  const int N = d->N, C = d->C;
+  const long long tok = (long long)B * S * C, fr = (long long)B * L;
+  int rc;
   StageScope sc(ST_TAIL, st);
-  if (d->num_blocks == 0) {
-    set_error("tensor engine needs at least one dual-path block");
-    return -1;
-  }
   float* preds[2] = {s1_pred, s2_pred};
   if (d->kind != VATSS_KIND_DPTN_MASK) {
     // speaker split + overlap-add + post-conv + skip + decoder projection: one gather over PReLU(x) (fp16) and enc
-    rc = launch_tail_fused(w.xa16, w.enc32, p.w2, p.c2, p.wdT, p.cfold, B, S, C, d->P, L, N, d->K, w.proj, st);
+    rc = launch_tail_fused(x16, enc32, p.w2, p.c2, p.wdT, p.cfold, B, S, C, d->P, L, N, d->K, w.proj, st);
     if (rc < 0) return rc;
     if (rc == 0) {
       for (int j = 0; j < 2; ++j)
@@ -328,19 +339,10 @@ int tensor_engine_forward(const vatss_model_desc* d, const float* const* params,
       return 0;
     }
   }
-  if ((rc = launch_tc_gemm(TC_EPI_F32, w.xa16, N, p.wspk, params[VATSS_P_SPK_B], nullptr, 0, nullptr, nullptr, w.y32,
+  // no fused instance for (N, K), or the masking head: speaker split, overlap-add and head as separate passes
+  if ((rc = launch_tc_gemm(TC_EPI_F32, x16, N, p.wspk, params[VATSS_P_SPK_B], nullptr, 0, nullptr, nullptr, w.y32,
                            2 * N, nullptr, 0, 0, nullptr, tok, 2 * N, N, st)))
     return rc;
-  if (d->kind != VATSS_KIND_DPTN_MASK) {
-    // overlap-add + post-conv + skip + decoder projection in one pass over the speaker-split output
-    rc = launch_ola_decode(w.y32, w.enc32, p.wfold, p.wdT, p.cfold, B, S, C, d->P, L, N, d->K, w.proj, st);
-    if (rc < 0) return rc;
-    if (rc == 0) {
-      for (int j = 0; j < 2; ++j)
-        if ((rc = launch_decoder_ola(w.proj + j * d->K, 2 * d->K, B, L, d->K, T, preds[j], st))) return rc;
-      return 0;
-    }
-  }
   if ((rc = launch_ola_token_major(w.y32, B, S, C, d->P, L, 2 * N, nullptr, w.ola16, st))) return rc;
   for (int j = 0; j < 2; ++j) {
     if (d->kind == VATSS_KIND_DPTN_MASK) {
@@ -350,9 +352,9 @@ int tensor_engine_forward(const vatss_model_desc* d, const float* const* params,
       if ((rc = launch_tc_gemm(TC_EPI_F32, w.ola16 + j * N, 2 * N, p.wgate, params[VATSS_P_HGATE_B], nullptr, 0, nullptr,
                                nullptr, w.hG, N, nullptr, 0, 0, nullptr, fr, N, N, st)))
         return rc;
-      if ((rc = launch_mask_combine(w.hT, w.hG, w.enc32, w.u32, fr * N, st))) return rc;
+      if ((rc = launch_mask_combine(w.hT, w.hG, enc32, w.u32, fr * N, st))) return rc;
     } else {
-      if ((rc = launch_tc_gemm(TC_EPI_F32, w.ola16 + j * N, 2 * N, p.whead, params[VATSS_P_HEAD_B], w.enc32, N, nullptr,
+      if ((rc = launch_tc_gemm(TC_EPI_F32, w.ola16 + j * N, 2 * N, p.whead, params[VATSS_P_HEAD_B], enc32, N, nullptr,
                                nullptr, w.u32, N, nullptr, 0, 0, nullptr, fr, N, N, st)))
         return rc;
     }

@@ -61,6 +61,11 @@ def test_bad_arguments_report_errors(lib):
     assert b"shorter than one chunk" in lib.vatss_last_error()
     assert lib.vatss_workspace_bytes(ctypes.byref(d), 4, 64000, 0) > 0
     assert lib.vatss_segment(None, 1, 1, 5, 10, 5, None, None) != 0
+    # no dual-path blocks: AUTO falls back to the generic engine and says why
+    assert lib.vatss_engine_fallback_reason(ctypes.byref(d)) is None
+    d.num_blocks = 0
+    assert b"no dual-path blocks" in lib.vatss_engine_fallback_reason(ctypes.byref(d))
+    assert lib.vatss_packed_weight_bytes(ctypes.byref(d)) == 0
 
 
 def test_state_dict_layout_and_init_match_reference_checksum(golden_dir):
