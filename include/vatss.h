@@ -219,6 +219,28 @@ int vatss_tc_tail(const vatss_model_desc* d, const float* const* params, int n_p
                   const void* x16, const float* enc, int B, int T, float* s1_pred, float* s2_pred,
                   void* workspace, size_t workspace_bytes, void* stream);
 
+/* Long recordings: overlapping windows separated as one batch, speaker order aligned between neighbouring windows and
+ * crossfaded back together.  No reference counterpart: the reference separates whole fixed-length clips.
+ * Geometry: window W samples, hop H with W/2 <= H < W, overlap O = W - H.  A recording of T samples has
+ * n = vatss_longform_windows(T, W, H) windows (1 if T <= W, else 1 + ceil((T - W) / H)); window j covers
+ * [jH, jH + W) and is zero at or past T.  Windows of R recordings are numbered w = r n + j. */
+int vatss_longform_windows(int T, int W, int H);   /* n, or <0 on bad arguments */
+/* Cut windows [first, first + count) of mix (R,T) into mix_out (count,W).  emb1/emb2 (R,E,Tv) or NULL: also cut the
+ * embedding windows emb*_out (count,E,W/spf), window j taking frames [jH/spf, jH/spf + W/spf) with frames at or past
+ * Tv repeating frame Tv-1 (spf = samples per video frame; W and H must be multiples of it). */
+int vatss_window_cut(const float* mix, const float* emb1, const float* emb2, int R, int T, int Tv, int E, int W, int H,
+                     int spf, int first, int count, float* mix_out, float* emb1_out, float* emb2_out, void* stream);
+/* Bytes of scratch vatss_window_stitch needs for R recordings of n windows each (0 on bad arguments). */
+size_t vatss_window_stitch_scratch_bytes(int R, int n);
+/* y1, y2 (R n, W): the two speaker outputs of every window -> s1, s2 (R,T).  For each adjacent pair (r, j) the
+ * overlap's fp64 sums [a1.b1, a1.b2, a2.b1, a2.b2, a1.a1, a2.a2, b1.b1, b2.b2] (a = window j from offset H, b = window
+ * j+1 from offset 0) decide a swap when cos(a1,b2) + cos(a2,b1) > cos(a1,b1) + cos(a2,b2) (normalised correlation, 0
+ * for a zero energy); window j then gives speaker s from its row s XOR (flags 0..j-1 XORed), so the output keeps
+ * window 0's order.  In an overlap, position i in [0,O): (1 - a) y_j + a y_{j+1}, a = (i + 0.5) / O in fp32.
+ * swaps_out (R, n-1) u8 and corr_out (R, n-1, 8) f64 may be NULL.  Bitwise reproducible. */
+int vatss_window_stitch(const float* y1, const float* y2, int R, int T, int W, int H, float* s1, float* s2,
+                        uint8_t* swaps_out, double* corr_out, void* scratch, size_t scratch_bytes, void* stream);
+
 /* Instrumentation (no reference counterpart; used by bench.py).
  * vatss_launch_count: number of kernels this library has launched in this process.
  * vatss_profile_begin: start recording CUDA-event pairs around the stages of subsequent calls

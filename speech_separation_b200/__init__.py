@@ -7,6 +7,7 @@ hand-written CUDA kernels inside libvatss_b200.so (C ABI in include/vatss.h).
 from .data import SSDataset, collate_fn, make_dataloader
 from .inference import Inferencer, MetricTracker
 from .lipreader import Lipreading, extract_embeddings, init_lipreader, make_embeddings
+from .longform import LongFormSeparator
 from .loss import SiSNRLoss, SiSNRWavLoss, pit_sisnr_all
 from .metrics import SISNRiMetric, SISNRMetric
 from .model import DPRNNEncDec, DPTNAVWavEncDec, DPTNEncDec, DPTNWavEncDec, OverlapAdd, SplitToFolds
@@ -14,5 +15,5 @@ from .model import DPRNNEncDec, DPTNAVWavEncDec, DPTNEncDec, DPTNWavEncDec, Over
 __all__ = [
     "DPTNAVWavEncDec", "DPTNWavEncDec", "DPTNEncDec", "DPRNNEncDec", "SplitToFolds", "OverlapAdd",
     "SiSNRLoss", "SiSNRWavLoss", "SISNRMetric", "SISNRiMetric", "pit_sisnr_all", "Inferencer", "MetricTracker", "SSDataset", "collate_fn", "make_dataloader",
-    "Lipreading", "init_lipreader", "extract_embeddings", "make_embeddings",
+    "Lipreading", "init_lipreader", "extract_embeddings", "make_embeddings", "LongFormSeparator",
 ]

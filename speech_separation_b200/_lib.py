@@ -91,6 +91,11 @@ EXPORTS = {
     "vatss_sisnr_chunks": (ctypes.c_int, [ctypes.c_int]),
     "vatss_pit_sisnr": (ctypes.c_int, [ctypes.c_void_p] * 5 + [ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 5),
     "vatss_pit_sisnr_backward": (ctypes.c_int, [ctypes.c_void_p] * 4 + [ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 6),
+    "vatss_longform_windows": (ctypes.c_int, [ctypes.c_int] * 3),
+    "vatss_window_cut": (ctypes.c_int, [ctypes.c_void_p] * 3 + [ctypes.c_int] * 9 + [ctypes.c_void_p] * 4),
+    "vatss_window_stitch_scratch_bytes": (ctypes.c_size_t, [ctypes.c_int, ctypes.c_int]),
+    "vatss_window_stitch": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p] + [ctypes.c_int] * 4 +
+                            [ctypes.c_void_p] * 5 + [ctypes.c_size_t, ctypes.c_void_p]),
     "vatss_debug_lipreader": (None, [ctypes.c_int]),
     "vatss_debug_lipreader_kernel": (None, [ctypes.c_int]),
     "vatss_debug_lipreader_trace": (None, [ctypes.c_void_p]),

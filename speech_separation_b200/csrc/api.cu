@@ -502,6 +502,52 @@ int vatss_pit_sisnr_backward(const float* s1p, const float* s2p, const float* s1
                                    (cudaStream_t)stream);
 }
 
+static int check_longform(int T, int W, int H) {
+  VATSS_CHECK_ARG(T > 0 && W > 0, "longform: empty recording or window (T=%d, W=%d)", T, W);
+  VATSS_CHECK_ARG(2 * (long long)H >= W && H < W, "longform: hop %d must satisfy W/2 <= hop < W (W=%d)", H, W);
+  return 0;
+}
+
+int vatss_longform_windows(int T, int W, int H) {
+  if (check_longform(T, W, H)) return -1;
+  return longform_windows(T, W, H);
+}
+
+int vatss_window_cut(const float* mix, const float* emb1, const float* emb2, int R, int T, int Tv, int E, int W, int H,
+                     int spf, int first, int count, float* mix_out, float* emb1_out, float* emb2_out, void* stream) {
+  if (check_longform(T, W, H)) return -1;
+  VATSS_CHECK_ARG(mix && mix_out, "window_cut: NULL pointer");
+  VATSS_CHECK_ARG(R > 0 && R <= 65535, "window_cut: R=%d recordings out of range", R);
+  const long long total = (long long)R * longform_windows(T, W, H);
+  VATSS_CHECK_ARG(first >= 0 && count >= 0 && count <= 65535 && first + (long long)count <= total,
+                  "window_cut: windows [%d, %d + %d) outside [0, %lld)", first, first, count, total);
+  VATSS_CHECK_ARG((emb1 == nullptr) == (emb2 == nullptr) && (emb1 == nullptr) == (emb1_out == nullptr) &&
+                      (emb1_out == nullptr) == (emb2_out == nullptr),
+                  "window_cut: give both embeddings and both embedding outputs, or none");
+  if (emb1) {
+    VATSS_CHECK_ARG(E > 0 && Tv > 0, "window_cut: E=%d, Tv=%d must be positive", E, Tv);
+    VATSS_CHECK_ARG(spf > 0 && W % spf == 0 && H % spf == 0,
+                    "window_cut: window %d and hop %d must be multiples of samples_per_video_frame %d", W, H, spf);
+  }
+  return launch_window_cut(mix, emb1, emb2, R, T, Tv, E, W, H, spf, first, count, mix_out, emb1_out, emb2_out,
+                           (cudaStream_t)stream);
+}
+
+size_t vatss_window_stitch_scratch_bytes(int R, int n) { return window_stitch_scratch_bytes(R, n); }
+
+int vatss_window_stitch(const float* y1, const float* y2, int R, int T, int W, int H, float* s1, float* s2,
+                        uint8_t* swaps_out, double* corr_out, void* scratch, size_t scratch_bytes, void* stream) {
+  if (check_longform(T, W, H)) return -1;
+  VATSS_CHECK_ARG(y1 && y2 && s1 && s2 && scratch, "window_stitch: NULL pointer");
+  VATSS_CHECK_ARG(R > 0 && R <= 65535, "window_stitch: R=%d recordings out of range", R);
+  const int n = longform_windows(T, W, H);
+  VATSS_CHECK_ARG((long long)R * n < (1ll << 31), "window_stitch: %d x %d windows", R, n);
+  const size_t need = window_stitch_scratch_bytes(R, n);
+  VATSS_CHECK_ARG(scratch_bytes >= need, "window_stitch: scratch too small: %zu bytes given, %zu needed",
+                  scratch_bytes, need);
+  return launch_window_stitch(y1, y2, R, T, W, H, s1, s2, swaps_out, corr_out, scratch, (cudaStream_t)stream);
+}
+
 void vatss_debug_lipreader(int flags) { vatss::g_lip_dbg = flags; }
 void vatss_debug_lipreader_kernel(int version) { vatss::g_lip_tc_version = version == 2 ? 2 : 1; }
 void vatss_debug_lipreader_trace(void* dev_buffer) { vatss::g_lip_trace = (long long*)dev_buffer; }

@@ -154,4 +154,12 @@ int launch_pit_sisnr_backward(const float* s1p, const float* s2p, const float* s
                               const double* scratch, const double* summary, const float* grad_out, float* g1, float* g2,
                               cudaStream_t st);
 
+// longform.cu
+int longform_windows(int T, int W, int H);
+size_t window_stitch_scratch_bytes(int R, int n);
+int launch_window_cut(const float* mix, const float* e1, const float* e2, int R, int T, int Tv, int E, int W, int H,
+                      int spf, int first, int count, float* mix_out, float* e1_out, float* e2_out, cudaStream_t st);
+int launch_window_stitch(const float* y1, const float* y2, int R, int T, int W, int H, float* s1, float* s2,
+                         uint8_t* swaps_out, double* corr_out, void* scratch, cudaStream_t st);
+
 }  // namespace vatss

@@ -188,8 +188,16 @@ class _DualPathEncDec(nn.Module):
 
     def _run(self, mix, e1, e2):
         mix = _lib.f32c(mix, "mix")
+        return self._run_into(mix, e1, e2, torch.empty_like(mix), torch.empty_like(mix))
+
+    def _run_into(self, mix, e1, e2, s1, s2):
+        """The forward with caller-provided outputs: s1, s2 contiguous float32 (B, T) on mix's device."""
+        mix = _lib.f32c(mix, "mix")
         if mix.dim() != 2:
             raise ValueError(f"mix must be (batch, time), got {tuple(mix.shape)}")
+        for t, name in ((s1, "s1"), (s2, "s2")):
+            if t.shape != mix.shape or t.dtype != torch.float32 or not t.is_contiguous() or t.device != mix.device:
+                raise ValueError(f"{name} output must be contiguous float32 {tuple(mix.shape)} on {mix.device}")
         B, T = mix.shape
         Tv = 0
         if self.KIND == "dptn_av":
@@ -202,8 +210,6 @@ class _DualPathEncDec(nn.Module):
         with torch.cuda.device(mix.device):
             lib = self._prepare(mix.device)
             ws = self._workspace(lib, B, T, Tv, mix.device)
-            s1 = torch.empty_like(mix)
-            s2 = torch.empty_like(mix)
             rc = lib.vatss_forward(ctypes.byref(self._desc), self._ptr_table, len(self._ptr_table),
                                    self._packed.data_ptr(), mix.data_ptr(),
                                    e1.data_ptr() if e1 is not None else None,
