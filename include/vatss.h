@@ -241,6 +241,21 @@ size_t vatss_window_stitch_scratch_bytes(int R, int n);
 int vatss_window_stitch(const float* y1, const float* y2, int R, int T, int W, int H, float* s1, float* s2,
                         uint8_t* swaps_out, double* corr_out, void* scratch, size_t scratch_bytes, void* stream);
 
+/* STOI / extended STOI of the four PIT pairings of a batch.  Replaces src/metrics/stoi.py (torchmetrics'
+ * ShortTimeObjectiveIntelligibility -> pystoi 0.4 stoi(target, preds, fs, extended) on the host, one utterance at a
+ * time) and the batch-level PIT of SS2BaseMetric.forward src/metrics/base_metric.py:53-60.  fp64 restatement:
+ * oracle/stoi_oracle.py (ESTOI without pystoi's EPS-scale noise, so deterministic).
+ * Workspace bytes for B utterances of T samples at fs Hz; 0 on bad arguments (B or T <= 0, fs outside
+ * 1 .. 1000000, or a signal shorter than one 256-sample frame after resampling to 10 kHz), see vatss_last_error. */
+size_t vatss_stoi_workspace_bytes(int B, int T, int fs);
+/* s1p, s2p, s1, s2 (B,T) f32 at fs Hz -> rows_out (B,4) f64: [s1p.s1, s2p.s2, s1p.s2, s2p.s1] (target second);
+ * kept_out (B,2) int32 or NULL: frames kept by the silent-frame removal of s1 and s2; summary_out (3,) f64:
+ * [batch mean of (row0 + row1)/2, batch mean of (row2 + row3)/2, max of the two].  extended = 1 gives ESTOI.
+ * No host synchronisation; bitwise reproducible and independent of the other utterances of the batch. */
+int vatss_stoi(const float* s1p, const float* s2p, const float* s1, const float* s2, int B, int T, int fs, int extended,
+               double* rows_out, int* kept_out, double* summary_out, void* workspace, size_t workspace_bytes,
+               void* stream);
+
 /* Instrumentation (no reference counterpart; used by bench.py).
  * vatss_launch_count: number of kernels this library has launched in this process.
  * vatss_profile_begin: start recording CUDA-event pairs around the stages of subsequent calls

@@ -96,6 +96,9 @@ EXPORTS = {
     "vatss_window_stitch_scratch_bytes": (ctypes.c_size_t, [ctypes.c_int, ctypes.c_int]),
     "vatss_window_stitch": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p] + [ctypes.c_int] * 4 +
                             [ctypes.c_void_p] * 5 + [ctypes.c_size_t, ctypes.c_void_p]),
+    "vatss_stoi_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int] * 3),
+    "vatss_stoi": (ctypes.c_int, [ctypes.c_void_p] * 4 + [ctypes.c_int] * 4 + [ctypes.c_void_p] * 4 +
+                   [ctypes.c_size_t, ctypes.c_void_p]),
     "vatss_debug_lipreader": (None, [ctypes.c_int]),
     "vatss_debug_lipreader_kernel": (None, [ctypes.c_int]),
     "vatss_debug_lipreader_trace": (None, [ctypes.c_void_p]),

@@ -548,6 +548,16 @@ int vatss_window_stitch(const float* y1, const float* y2, int R, int T, int W, i
   return launch_window_stitch(y1, y2, R, T, W, H, s1, s2, swaps_out, corr_out, scratch, (cudaStream_t)stream);
 }
 
+size_t vatss_stoi_workspace_bytes(int B, int T, int fs) { return stoi_workspace_bytes(B, T, fs); }
+
+int vatss_stoi(const float* s1p, const float* s2p, const float* s1, const float* s2, int B, int T, int fs, int extended,
+               double* rows_out, int* kept_out, double* summary_out, void* workspace, size_t workspace_bytes,
+               void* stream) {
+  VATSS_CHECK_ARG(s1p && s2p && s1 && s2 && rows_out && summary_out && workspace, "stoi: NULL pointer");
+  return launch_stoi(s1p, s2p, s1, s2, B, T, fs, extended, rows_out, kept_out, summary_out, workspace,
+                     workspace_bytes, (cudaStream_t)stream);
+}
+
 void vatss_debug_lipreader(int flags) { vatss::g_lip_dbg = flags; }
 void vatss_debug_lipreader_kernel(int version) { vatss::g_lip_tc_version = version == 2 ? 2 : 1; }
 void vatss_debug_lipreader_trace(void* dev_buffer) { vatss::g_lip_trace = (long long*)dev_buffer; }

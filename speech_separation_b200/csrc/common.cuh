@@ -162,4 +162,10 @@ int launch_window_cut(const float* mix, const float* e1, const float* e2, int R,
 int launch_window_stitch(const float* y1, const float* y2, int R, int T, int W, int H, float* s1, float* s2,
                          uint8_t* swaps_out, double* corr_out, void* scratch, cudaStream_t st);
 
+// stoi.cu
+size_t stoi_workspace_bytes(int B, int T, int fs);
+int launch_stoi(const float* s1p, const float* s2p, const float* s1, const float* s2, int B, int T, int fs,
+                int extended, double* rows, int* kept_out, double* summary, void* workspace, size_t bytes,
+                cudaStream_t st);
+
 }  // namespace vatss
