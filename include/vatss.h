@@ -317,6 +317,13 @@ void vatss_debug_lipreader_kernel(int version);
 /* debug: device buffer (>= 8192 int64) receiving globaltimer / clock64 stamps of the first 1024 CTAs of every
  * following tcgen05 convolution launch (the last launch wins); NULL disables */
 void vatss_debug_lipreader_trace(void* dev_buffer);
+/* debug: device pointers receiving every stage of the following lipreader forwards (NULL entries skipped; NULL / 0 disables).
+ * Slot 0: front end before the max pool (F, H1, W1, 64); slot 1: pooled trunk input (F, H0, W0, 64); block k = 0..7:
+ * slot 2+3k conv1 output after its activation, 3+3k shortcut output (blocks with a shortcut convolution only), 4+3k block
+ * output act(conv2 + residual).  Every slot holds all F = B T frames, fp32 under the f32 engine, fp16 under the tensor
+ * engine.  The table is copied at the call. */
+#define VATSS_LIP_NSTAGES 26
+void vatss_debug_lipreader_capture(void* const* stages, int n);
 size_t vatss_lipreader_packed_bytes(void);
 /* scratch for B x T frames cropped to Hc x Wc (frames are processed in chunks, so this is bounded) */
 size_t vatss_lipreader_workspace_bytes(int B, int T, int Hc, int Wc);

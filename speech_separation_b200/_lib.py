@@ -102,6 +102,7 @@ EXPORTS = {
     "vatss_debug_lipreader": (None, [ctypes.c_int]),
     "vatss_debug_lipreader_kernel": (None, [ctypes.c_int]),
     "vatss_debug_lipreader_trace": (None, [ctypes.c_void_p]),
+    "vatss_debug_lipreader_capture": (None, [ctypes.POINTER(ctypes.c_void_p), ctypes.c_int]),
     "vatss_lipreader_packed_bytes": (ctypes.c_size_t, []),
     "vatss_lipreader_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int] * 4),
     "vatss_lipreader_pack_weights": (ctypes.c_int, [ctypes.POINTER(ctypes.c_void_p), ctypes.c_int, ctypes.c_int,

@@ -561,6 +561,10 @@ int vatss_stoi(const float* s1p, const float* s2p, const float* s1, const float*
 void vatss_debug_lipreader(int flags) { vatss::g_lip_dbg = flags; }
 void vatss_debug_lipreader_kernel(int version) { vatss::g_lip_tc_version = version == 2 ? 2 : 1; }
 void vatss_debug_lipreader_trace(void* dev_buffer) { vatss::g_lip_trace = (long long*)dev_buffer; }
+void vatss_debug_lipreader_capture(void* const* stages, int n) {
+  static_assert(vatss::LIP_NSTAGES == VATSS_LIP_NSTAGES, "stage count");
+  for (int i = 0; i < vatss::LIP_NSTAGES; ++i) vatss::g_lip_capture[i] = (stages && i < n) ? stages[i] : nullptr;
+}
 size_t vatss_lipreader_packed_bytes(void) { return lip_packed_bytes(); }
 size_t vatss_lipreader_workspace_bytes(int B, int T, int Hc, int Wc) { return lip_workspace_bytes(B, T, Hc, Wc); }
 int vatss_lipreader_pack_weights(const float* const* params, int n_params, int relu_type, void* packed,

@@ -478,19 +478,32 @@ int lip_geometry(int Hc, int Wc, LipGeom* g) {
   return 0;
 }
 
+// Per-frame pitch of each of the four trunk buffers: the largest trunk activation, max over layers of H_l W_l C_l.
+// Layer 1 (H0 W0 64) for most crops, but layer 4 (H3 W3 512) for crops with a side of 8 - 12 pixels (8 x 8: 256 < 512).
+static long long lip_trunk_frame_floats(const LipGeom& g) {
+  long long m = 0;
+  for (int l = 0; l < 4; ++l) {
+    const long long v = (long long)g.H[l] * g.W[l] * (64 << l);
+    m = v > m ? v : m;
+  }
+  return m;
+}
+
 static long long lip_frame_floats(const LipGeom& g) {
-  // conv3d output + four trunk buffers of the largest trunk activation (layer1: H0 x W0 x 64)
-  return (long long)g.H1 * g.W1 * 64 + 4ll * g.H[0] * g.W[0] * 64;
+  // conv3d output + four trunk buffers
+  return (long long)g.H1 * g.W1 * 64 + 4ll * lip_trunk_frame_floats(g);
 }
 
 int lip_chunk_frames(long long F) { return (int)(F < LIP_CHUNK ? F : LIP_CHUNK); }
+
+void* g_lip_capture[LIP_NSTAGES] = {};
 
 size_t lip_workspace_bytes(int B, int T, int Hc, int Wc) {
   LipGeom g;
   if (B <= 0 || T <= 0 || lip_geometry(Hc, Wc, &g)) return 0;
   const long long fc = lip_chunk_frames((long long)B * T);
   // fp32 buffers + fp16 shadows of the trunk buffers and the front end's im2col matrix (tensor engine) + slack
-  return (size_t)(fc * lip_frame_floats(g) * 4 + fc * 4ll * g.H[0] * g.W[0] * 64 * 2 +
+  return (size_t)(fc * lip_frame_floats(g) * 4 + fc * 4ll * lip_trunk_frame_floats(g) * 2 +
                   fc * (long long)g.H1 * g.W1 * LIP_FRONT_K * 2 + 4096);
 }
 
@@ -514,7 +527,7 @@ int lip_forward(const void* packed, size_t packed_bytes, int relu_type, const fl
   const long long F = (long long)B * T;
   const int FC = lip_chunk_frames(F);
   float* buf0 = (float*)workspace;
-  const long long trunk_floats = (long long)FC * g.H[0] * g.W[0] * 64;
+  const long long trunk_floats = (long long)FC * lip_trunk_frame_floats(g);
   float* tb[4];
   for (int i = 0; i < 4; ++i) tb[i] = buf0 + (long long)FC * g.H1 * g.W1 * 64 + i * trunk_floats;
   __half* tb16[4];
@@ -536,6 +549,14 @@ int lip_forward(const void* packed, size_t packed_bytes, int relu_type, const fl
   for (long long f0 = 0; f0 < F; f0 += FC) {
     const int nf = (int)((F - f0) < FC ? (F - f0) : FC);
     const bool tc = engine == VATSS_LIP_ENGINE_TENSOR;
+    // debug (vatss_debug_lipreader_capture): copy the stage just produced, (nf, per_frame) values, to its capture slot
+    auto capture = [&](int slot, const void* src, long long per_frame) -> int {
+      if (!g_lip_capture[slot]) return 0;
+      const long long esz = tc ? (long long)sizeof(__half) : (long long)sizeof(float);
+      VATSS_CUDA_OK(cudaMemcpyAsync((char*)g_lip_capture[slot] + f0 * per_frame * esz, src, nf * per_frame * esz,
+                                    cudaMemcpyDeviceToDevice, st));
+      return 0;
+    };
     LipFrontArgs a;
     a.vid = video; a.B = B; a.T = T; a.Hin = Hin; a.Win = Win; a.y0 = y0; a.x0 = x0; a.Hc = Hc; a.Wc = Wc;
     a.H1 = g.H1; a.W1 = g.W1; a.pre_scale = pre_scale; a.pre_shift = pre_shift;
@@ -553,14 +574,18 @@ int lip_forward(const void* packed, size_t packed_bytes, int relu_type, const fl
       cf.taps = 1; cf.cin = LIP_FRONT_K; cf.ks = 1; cf.stride = 1; cf.pad = 0;
       __half* front16 = (__half*)buf0;   // (nf, H1, W1, 64) fp16 in the (unused) fp32 front-end buffer
       if (int rc = lip_conv_tc(pk, cf, im2col16, nf, g.H1, g.W1, g.H1, g.W1, nullptr, relu_type, front16, st)) return rc;
+      if (int rc = capture(0, front16, (long long)g.H1 * g.W1 * 64)) return rc;
       k_lip_maxpool<__half><<<pool_grid, 256, 0, st>>>(front16, nf, g.H1, g.W1, 64, g.H[0], g.W[0], nullptr, tb16[0]);
       VATSS_LAUNCH_OK();
+      if (int rc = capture(1, tb16[0], (long long)g.H[0] * g.W[0] * 64)) return rc;
     } else {
       const int slots = 2 * num_sms();
       k_lip_front3d<<<items < slots ? items : slots, 192, front_smem, st>>>(a);
       VATSS_LAUNCH_OK();
+      if (int rc = capture(0, buf0, (long long)g.H1 * g.W1 * 64)) return rc;
       k_lip_maxpool<float><<<pool_grid, 256, 0, st>>>(buf0, nf, g.H1, g.W1, 64, g.H[0], g.W[0], tb[0], nullptr);
       VATSS_LAUNCH_OK();
+      if (int rc = capture(1, tb[0], (long long)g.H[0] * g.W[0] * 64)) return rc;
     }
     int cur = 0, H = g.H[0], W = g.W[0], ci = 1, final_c = 64;
     for (int l = 0; l < 4; ++l)
@@ -568,17 +593,22 @@ int lip_forward(const void* packed, size_t packed_bytes, int relu_type, const fl
         const LipConv &c1 = t[ci], &c2 = t[ci + 1], &cs = t[ci + 2];
         const int Ho = out_dim(H, 3, c1.stride, 1), Wo = out_dim(W, 3, c1.stride, 1);
         const int xb = cur, tbuf = (cur + 1) & 3, rb = (cur + 2) & 3, yb = (cur + 3) & 3;
+        const int k = 2 * l + b;
+        const long long out_frame = (long long)Ho * Wo * c1.cout;
         if (tc) {
           int rc = lip_conv_tc(pk, c1, tb16[xb], nf, H, W, Ho, Wo, nullptr, relu_type, tb16[tbuf], st);
           if (rc) return rc;
+          if ((rc = capture(2 + 3 * k, tb16[tbuf], out_frame))) return rc;
           const __half* res = tb16[xb];
           if (cs.cout) {
             rc = lip_conv_tc(pk, cs, tb16[xb], nf, H, W, Ho, Wo, nullptr, LIP_ACT_NONE, tb16[rb], st);
             if (rc) return rc;
+            if ((rc = capture(3 + 3 * k, tb16[rb], out_frame))) return rc;
             res = tb16[rb];
           }
           rc = lip_conv_tc(pk, c2, tb16[tbuf], nf, Ho, Wo, Ho, Wo, res, relu_type, tb16[yb], st);
           if (rc) return rc;
+          if ((rc = capture(4 + 3 * k, tb16[yb], out_frame))) return rc;
         } else {
           auto run = [&](const LipConv& c, const float* in, int Hi, int Wi, const float* res, int act, float* o) -> int {
             LipConvArgs a;
@@ -593,12 +623,15 @@ int lip_forward(const void* packed, size_t packed_bytes, int relu_type, const fl
             return 0;
           };
           if (int rc = run(c1, tb[xb], H, W, nullptr, relu_type, tb[tbuf])) return rc;
+          if (int rc = capture(2 + 3 * k, tb[tbuf], out_frame)) return rc;
           const float* res = tb[xb];
           if (cs.cout) {
             if (int rc = run(cs, tb[xb], H, W, nullptr, LIP_ACT_NONE, tb[rb])) return rc;
+            if (int rc = capture(3 + 3 * k, tb[rb], out_frame)) return rc;
             res = tb[rb];
           }
           if (int rc = run(c2, tb[tbuf], Ho, Wo, res, relu_type, tb[yb])) return rc;
+          if (int rc = capture(4 + 3 * k, tb[yb], out_frame)) return rc;
         }
         cur = yb; H = Ho; W = Wo; final_c = c2.cout;
       }

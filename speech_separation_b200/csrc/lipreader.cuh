@@ -29,6 +29,8 @@ int lip_forward(const void* packed, size_t packed_bytes, int relu_type, const fl
 extern long long* g_lip_trace;
 extern int g_lip_tc_version;
 extern int g_lip_dbg;   // experiment switches of k_lip_conv_tc (0 in production)
+constexpr int LIP_NSTAGES = 26;   // front end, pooled input, 8 blocks x (conv1, shortcut, output): VATSS_LIP_NSTAGES
+extern void* g_lip_capture[LIP_NSTAGES];   // debug: per-stage copies of the next forwards (all NULL in production)
 
 // tcgen05 engine: out16 (F, Ho, Wo, Cout) = act(conv(in16 (F, H, W, Cin)) * scale + shift + res16), fp16 activations,
 // fp32 accumulation in TMEM

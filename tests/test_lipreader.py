@@ -164,11 +164,13 @@ def test_cuda_utterance_boundaries_and_frame_chunks():
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("B,T,H,W", [(1, 1, 88, 88), (2, 2, 70, 58), (1, 3, 33, 87), (3, 4, 16, 8)])
+@pytest.mark.parametrize("B,T,H,W", [(1, 1, 88, 88), (2, 2, 70, 58), (1, 3, 33, 87), (3, 4, 16, 8), (2, 3, 8, 8),
+                                     (1, 4, 12, 8), (2, 2, 8, 11)])
 def test_cuda_odd_geometries_and_short_clips(B, T, H, W):
     """Shapes the production pipeline never produces but the reference class accepts: a single frame (all temporal taps
     but one fall into the zero padding), odd widths after every stride-2 stage (58 -> 29 -> 15 -> 8 -> 4 -> 2), ragged last
-    row tiles, images smaller than a convolution tile - against the CPU oracle, both engines."""
+    row tiles, images smaller than a convolution tile, and crops of 8 - 12 pixels on a side, where layer 4 (1 x 1 x 512)
+    is the largest trunk activation - against the CPU oracle, both engines."""
     relu_type = "prelu"
     sd = LO.make_state_dict(relu_type, 21)
     rng = np.random.Generator(np.random.PCG64(B * 1000 + T * 100 + H + W))
