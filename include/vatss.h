@@ -170,6 +170,30 @@ int vatss_pit_sisnr(const float* s1p, const float* s2p, const float* s1, const f
                     const float* mix, int B, int T, double* rows_out, double* rows_loss_out,
                     double* summary_out, double* scratch, void* stream);
 
+/* PIT SI-SDR: torchmetrics' ScaleInvariantSignalDistortionRatio (which src/metrics/si_sdr.py wraps, zero_mean=False by
+ * default) with the batch-level PIT of SS2BaseMetric.forward src/metrics/base_metric.py:53-60.  Same inputs, row order
+ * and scratch (B*chunks*16 doubles) as vatss_pit_sisnr; one pass over the waveforms.  Per pair, in fp64 from the raw
+ * moments: alpha = (<p,t> + eps) / (||t||^2 + eps), 10 log10((||alpha t||^2 + eps) / (||alpha t - p||^2 + eps)),
+ * eps = FLT_EPSILON; zero_mean = 1 removes the means first.  rows_out (B,6) f64 (rows 4, 5 NaN when mix is NULL);
+ * summary_out (7) f64: [mean (r0+r1)/2, mean (r2+r3)/2, max of the two, SI-SDRi = max - mean (r4+r5)/2, mean r4,
+ * mean r5, B] (3..5 NaN when mix is NULL).  fp64 restatement: oracle/sdr_oracle.py. */
+int vatss_pit_sisdr(const float* s1p, const float* s2p, const float* s1, const float* s2, const float* mix, int B,
+                    int T, int zero_mean, double* rows_out, double* summary_out, double* scratch, void* stream);
+
+/* PIT SDR / SDRi: BSS-eval SDR with a distortion filter of filter_length taps (torchmetrics' SignalDistortionRatio on
+ * its direct-solve path) for the six pairings of vatss_pit_sisnr, and the summary of vatss_pit_sisdr.  Per pair, in
+ * fp64: optional mean removal, both signals normalised by max(||x||, 1e-6), r[l] = sum t[n] t[n+l] and
+ * b[l] = sum t[n] p[n+l] for l < filter_length (direct lag sums), r[0] += load_diag (load_diag < 0: none), the
+ * symmetric Toeplitz system R x = b solved by the Levinson recursion, coh = b.x, 10 log10(coh / (1 - coh)).  A target
+ * whose recursion meets a prediction error <= 0 (all zeros, or a singular R without load_diag) gets NaN rows.
+ * Workspace bytes for B utterances of T samples; 0 on bad arguments (B or T <= 0, B > 65535, filter_length < 1 or
+ * above 2048, T < filter_length), see vatss_last_error.  No host synchronisation; bitwise reproducible, and an
+ * utterance gets the same rows alone as inside a batch.  fp64 restatement: oracle/sdr_oracle.py. */
+size_t vatss_sdr_workspace_bytes(int B, int T, int filter_length);
+int vatss_sdr(const float* s1p, const float* s2p, const float* s1, const float* s2, const float* mix, int B, int T,
+              int filter_length, int zero_mean, double load_diag, double* rows_out, double* summary_out,
+              void* workspace, size_t workspace_bytes, void* stream);
+
 /* Gradient of summary_out[0] (the batch-level PIT loss) with respect to the two predictions: the first piece of the
  * reference's training step (`batch["loss"].backward()`, src/trainer/trainer.py:46, through BaseSSLoss.forward
  * src/loss/ss_losses.py:10-26 and SiSNRLoss.forward :100-114).  `scratch` and `summary` are those a preceding

@@ -90,6 +90,10 @@ EXPORTS = {
     "vatss_profile_end": (ctypes.c_int, [ctypes.POINTER(ctypes.c_float), ctypes.POINTER(ctypes.c_int), ctypes.c_int]),
     "vatss_sisnr_chunks": (ctypes.c_int, [ctypes.c_int]),
     "vatss_pit_sisnr": (ctypes.c_int, [ctypes.c_void_p] * 5 + [ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 5),
+    "vatss_pit_sisdr": (ctypes.c_int, [ctypes.c_void_p] * 5 + [ctypes.c_int] * 3 + [ctypes.c_void_p] * 4),
+    "vatss_sdr_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int] * 3),
+    "vatss_sdr": (ctypes.c_int, [ctypes.c_void_p] * 5 + [ctypes.c_int] * 4 + [ctypes.c_double] + [ctypes.c_void_p] * 3 +
+                  [ctypes.c_size_t, ctypes.c_void_p]),
     "vatss_pit_sisnr_backward": (ctypes.c_int, [ctypes.c_void_p] * 4 + [ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 6),
     "vatss_longform_windows": (ctypes.c_int, [ctypes.c_int] * 3),
     "vatss_window_cut": (ctypes.c_int, [ctypes.c_void_p] * 3 + [ctypes.c_int] * 9 + [ctypes.c_void_p] * 4),

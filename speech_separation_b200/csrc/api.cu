@@ -502,6 +502,22 @@ int vatss_pit_sisnr_backward(const float* s1p, const float* s2p, const float* s1
                                    (cudaStream_t)stream);
 }
 
+int vatss_pit_sisdr(const float* s1p, const float* s2p, const float* s1, const float* s2, const float* mix, int B,
+                    int T, int zero_mean, double* rows_out, double* summary_out, double* scratch, void* stream) {
+  VATSS_CHECK_ARG(s1p && s2p && s1 && s2 && rows_out && summary_out && scratch, "pit_sisdr: NULL pointer");
+  return launch_pit_sisdr(s1p, s2p, s1, s2, mix, B, T, zero_mean, rows_out, summary_out, scratch, (cudaStream_t)stream);
+}
+
+size_t vatss_sdr_workspace_bytes(int B, int T, int filter_length) { return sdr_workspace_bytes(B, T, filter_length); }
+
+int vatss_sdr(const float* s1p, const float* s2p, const float* s1, const float* s2, const float* mix, int B, int T,
+              int filter_length, int zero_mean, double load_diag, double* rows_out, double* summary_out,
+              void* workspace, size_t workspace_bytes, void* stream) {
+  VATSS_CHECK_ARG(s1p && s2p && s1 && s2 && rows_out && summary_out && workspace, "sdr: NULL pointer");
+  return launch_sdr(s1p, s2p, s1, s2, mix, B, T, filter_length, zero_mean, load_diag, rows_out, summary_out, workspace,
+                    workspace_bytes, (cudaStream_t)stream);
+}
+
 static int check_longform(int T, int W, int H) {
   VATSS_CHECK_ARG(T > 0 && W > 0, "longform: empty recording or window (T=%d, W=%d)", T, W);
   VATSS_CHECK_ARG(2 * (long long)H >= W && H < W, "longform: hop %d must satisfy W/2 <= hop < W (W=%d)", H, W);

@@ -162,6 +162,42 @@ int launch_window_cut(const float* mix, const float* e1, const float* e2, int R,
 int launch_window_stitch(const float* y1, const float* y2, int R, int T, int W, int H, float* s1, float* s2,
                          uint8_t* swaps_out, double* corr_out, void* scratch, cudaStream_t st);
 
+// sisnr.cu: the 16 raw fp64 moments per chunk of k_sisnr_moments, B * sisnr_chunks(T) * 16 doubles
+int launch_sisnr_moments(const float* s1p, const float* s2p, const float* s1, const float* s2, const float* mix, int B,
+                         int T, double* scratch, cudaStream_t st);
+int launch_pit_sisdr(const float* s1p, const float* s2p, const float* s1, const float* s2, const float* mix, int B,
+                     int T, int zero_mean, double* rows, double* summary, double* scratch, cudaStream_t st);
+
+// Batch-level PIT summary of per-utterance rows (B,6) [s1p.s1, s2p.s2, s1p.s2, s2p.s1, mix.s1, mix.s2] (one thread):
+// [mean (r0+r1)/2, mean (r2+r3)/2, max of the two, max - mean (r4+r5)/2, mean r4, mean r5, B]; 3..5 NaN without mix.
+__device__ __forceinline__ void pit_summary7(const double* rows, int B, int has_mix, double* summary) {
+  double p1 = 0.0, p2 = 0.0, m1 = 0.0, m2 = 0.0;
+  for (int b = 0; b < B; ++b) {
+    p1 += (rows[6 * b] + rows[6 * b + 1]) * 0.5;
+    p2 += (rows[6 * b + 2] + rows[6 * b + 3]) * 0.5;
+    m1 += rows[6 * b + 4];
+    m2 += rows[6 * b + 5];
+  }
+  p1 /= (double)B;
+  p2 /= (double)B;
+  m1 /= (double)B;
+  m2 /= (double)B;
+  const double sep = p1 > p2 ? p1 : p2;   // Python max(perm_1, perm_2)
+  summary[0] = p1;
+  summary[1] = p2;
+  summary[2] = sep;
+  summary[3] = has_mix ? sep - (m1 + m2) * 0.5 : __longlong_as_double(0x7ff8000000000000ll);
+  summary[4] = has_mix ? m1 : __longlong_as_double(0x7ff8000000000000ll);
+  summary[5] = has_mix ? m2 : __longlong_as_double(0x7ff8000000000000ll);
+  summary[6] = (double)B;
+}
+
+// sdr.cu
+size_t sdr_workspace_bytes(int B, int T, int filter_length);
+int launch_sdr(const float* s1p, const float* s2p, const float* s1, const float* s2, const float* mix, int B, int T,
+               int filter_length, int zero_mean, double load_diag, double* rows, double* summary, void* workspace,
+               size_t bytes, cudaStream_t st);
+
 // stoi.cu
 size_t stoi_workspace_bytes(int B, int T, int fs);
 int launch_stoi(const float* s1p, const float* s2p, const float* s1, const float* s2, int B, int T, int fs,

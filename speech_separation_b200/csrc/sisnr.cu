@@ -143,6 +143,60 @@ int launch_pit_sisnr(const float* s1p, const float* s2p, const float* s1, const 
   return 0;
 }
 
+int launch_sisnr_moments(const float* s1p, const float* s2p, const float* s1, const float* s2, const float* mix, int B,
+                         int T, double* scratch, cudaStream_t st) {
+  const int chunks = sisnr_chunks(T);
+  k_sisnr_moments<<<dim3(chunks, B), 256, 0, st>>>(s1p, s2p, s1, s2, mix, T, chunks, scratch);
+  VATSS_LAUNCH_OK();
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------
+// SI-SDR (torchmetrics' scale_invariant_signal_distortion_ratio, which src/metrics/si_sdr.py wraps; zero_mean=False by
+// default) from the same raw moments: alpha = (<p,t> + eps) / (||t||^2 + eps), 10 log10((||alpha t||^2 + eps) /
+// (||alpha t - p||^2 + eps)), eps = FLT_EPSILON, both norms expanded in fp64.  zero_mean = 1 centres the moments first
+// (then the value is the SI-SNR of k_sisnr_finalize).  Rows 4, 5 are NaN without a mixture.
+// ------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+k_sisdr_finalize(const double* __restrict__ scratch, int B, int T, int chunks, int has_mix, int zero_mean,
+                 double* __restrict__ rows, double* __restrict__ summary) {
+  const double invT = zero_mean ? 1.0 / (double)T : 0.0;   // 0: the raw moments
+  const double eps = (double)FLT_EPSILON;
+  const int P_[6] = {0, 1, 0, 1, 4, 4};
+  const int G_[6] = {2, 3, 3, 2, 2, 3};
+  const int X_[6] = {10, 11, 12, 13, 14, 15};
+  for (int b = threadIdx.x; b < B; b += blockDim.x) {
+    double m[SISNR_NM];
+    for (int i = 0; i < SISNR_NM; ++i) m[i] = 0.0;
+    for (int c = 0; c < chunks; ++c)
+      for (int i = 0; i < SISNR_NM; ++i) m[i] += scratch[((size_t)b * chunks + c) * SISNR_NM + i];
+    for (int q = 0; q < 6; ++q) {
+      if (q >= 4 && !has_mix) {
+        rows[b * 6 + q] = __longlong_as_double(0x7ff8000000000000ll);
+        continue;
+      }
+      const PairMoments pm = centred(m, P_[q], G_[q], X_[q], invT);
+      const double alpha = (pm.dot + eps) / (pm.gg + eps);
+      const double sig = alpha * alpha * pm.gg;
+      double noise = sig - 2.0 * alpha * pm.dot + pm.pp;
+      if (noise < 0.0) noise = 0.0;
+      rows[b * 6 + q] = 10.0 * log10((sig + eps) / (noise + eps));
+    }
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) pit_summary7(rows, B, has_mix, summary);
+}
+
+int launch_pit_sisdr(const float* s1p, const float* s2p, const float* s1, const float* s2, const float* mix, int B,
+                     int T, int zero_mean, double* rows, double* summary, double* scratch, cudaStream_t st) {
+  VATSS_CHECK_ARG(B > 0 && T > 0, "pit_sisdr: empty batch (B=%d, T=%d)", B, T);
+  VATSS_CHECK_ARG(B <= 65535, "pit_sisdr: batch of %d utterances (at most 65535)", B);
+  if (int rc = launch_sisnr_moments(s1p, s2p, s1, s2, mix, B, T, scratch, st)) return rc;
+  k_sisdr_finalize<<<1, 256, 0, st>>>(scratch, B, T, sisnr_chunks(T), mix != nullptr, zero_mean, rows, summary);
+  VATSS_LAUNCH_OK();
+  return 0;
+}
+
 // ------------------------------------------------------------------------------------------
 // Backward of the batch-level PIT loss with respect to the two predictions (first piece of the training step,
 // src/trainer/trainer.py:46 `batch["loss"].backward()` through BaseSSLoss.forward src/loss/ss_losses.py:10-26).
