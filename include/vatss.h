@@ -34,7 +34,7 @@ extern "C" {
 #define VATSS_KIND_DPRNN 3     /* src/model/dprnn.py:230-276     DPRNNEncDec     */
 
 /* execution engines for the dual-path blocks (shape specialisation, not a backend switch):
- * GENERIC = fp32 SIMT kernels for any dimensions; TENSOR = tcgen05/TMEM kernels for the
+ * GENERIC = fp32 SIMT kernels for N <= 256, H <= 128, head dim <= 64 (W_hh in fp16 for H >= 108); TENSOR = tcgen05/TMEM kernels for the
  * production dimensions (N in {64,128}, H=128).  AUTO picks TENSOR when the shape allows. */
 #define VATSS_ENGINE_AUTO 0
 #define VATSS_ENGINE_GENERIC 1
@@ -233,6 +233,29 @@ int vatss_tc_lstm(const void* x16, const void* x16lo /* NULL, or half(x - half(x
  * pre-scaled by log2(e)/sqrt(hd); out16 (B*S*C, N).  mode 0 intra / 1 inter; force_simt=1 runs the SIMT fallback. */
 int vatss_tc_attention(const void* qkv16, void* out16, int mode, int B, int S, int C, int N, int heads, int force_simt,
                        void* stream);
+
+/* Stand-alone entry points of the GENERIC-engine kernels (fp32 SIMT; unit tests).  All tensors fp32.
+ * vatss_generic_gemm: out[m, n] (row pitch ldc) = act(A)[m, :] . W[n, :] + bias[n] + bias2[n] + R[m, n] for m < M,
+ *   n < NOUT; A (M, K) row pitch lda, W (NOUT, K) dense, R row pitch ldr; bias, bias2, R may be NULL;
+ *   act 0 none, 1 ReLU, 2 PReLU with slope *prelu_a (applied to A, as the speaker split does, dptn_wav.py:47-59). */
+int vatss_generic_gemm(const float* A, long long lda, const float* W, const float* bias, const float* bias2,
+                       const float* R, long long ldr, float* out, long long ldc, long long M, int NOUT, int K, int act,
+                       const float* prelu_a, void* stream);
+/* vatss_generic_layernorm: rows of N <= 256 features, dense; biased variance, eps 1e-5.
+ *   mode 0: out = LN(in + res) (src/model/dptn.py:47,51); mode 1: out = LN(in) + res (src/model/dprnn.py:42-45);
+ *   res may be NULL. */
+int vatss_generic_layernorm(const float* in, const float* res, const float* w, const float* b, float* out,
+                            long long rows, int N, int mode, void* stream);
+/* vatss_generic_attention: softmax(q k^T / sqrt(hd)) v per (sequence, head), hd = N / heads <= 64, any length;
+ * qkv (B*S*C, 3N) token-major, q unscaled (mha.in_proj output, src/model/dptn.py:16-21); out (B*S*C, N).
+ * mode 0 intra-chunk sequences, 1 inter-chunk. */
+int vatss_generic_attention(const float* qkv, float* out, int mode, int B, int S, int C, int N, int heads,
+                            void* stream);
+/* vatss_generic_lstm: the nn.LSTM recurrence (h0 = c0 = 0, gates i f g o) on pre (B*S*C, ndir*4H) = x W_ih^T + b_ih
+ * + b_hh of every direction; W_hh (4H, H) per direction (whh_r NULL for ndir = 1); out (B*S*C, ndir*H) = h.
+ * H a multiple of 4 up to 128; W_hh is used in fp32 for H <= 104 and rounded to fp16 for H >= 108. */
+int vatss_generic_lstm(const float* pre, const float* whh_f, const float* whh_r, float* out, int mode, int B, int S,
+                       int C, int H, int ndir, void* stream);
 
 /* vatss_tc_tail: the TENSOR engine's separator tail on its own - speaker split, overlap-add with the centred pad,
  * post-conv (or masking) head and decoder - through the same dispatch vatss_forward runs after its last block.

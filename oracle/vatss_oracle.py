@@ -184,11 +184,16 @@ def mha_self(z, P, pre, heads):
     q = q.reshape(G, Ls, heads, hd).transpose(0, 2, 1, 3)
     k = k.reshape(G, Ls, heads, hd).transpose(0, 2, 1, 3)
     v = v.reshape(G, Ls, heads, hd).transpose(0, 2, 1, 3)
-    s = (q @ k.transpose(0, 1, 3, 2)) / math.sqrt(hd)
-    s = s - s.max(axis=-1, keepdims=True)
-    p = np.exp(s)
-    p = p / p.sum(axis=-1, keepdims=True)
-    o = (p @ v).transpose(0, 2, 1, 3).reshape(G, Ls, N)
+    o = np.empty_like(q)
+    step = max(1, (1 << 24) // (heads * Ls * Ls))  # sequences per pass: score matrices of <= 128 MB in fp64
+    for g0 in range(0, G, step):
+        sl = slice(g0, g0 + step)
+        s = (q[sl] @ k[sl].transpose(0, 1, 3, 2)) / math.sqrt(hd)
+        s = s - s.max(axis=-1, keepdims=True)
+        p = np.exp(s)
+        p = p / p.sum(axis=-1, keepdims=True)
+        o[sl] = p @ v[sl]
+    o = o.transpose(0, 2, 1, 3).reshape(G, Ls, N)
     return o @ P[pre + "mha.out_proj.weight"].T + P[pre + "mha.out_proj.bias"]
 
 

@@ -73,7 +73,15 @@ EXPORTS = {
     "vatss_tc_lstm": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.POINTER(ctypes.c_void_p), ctypes.c_void_p] +
                       [ctypes.c_int] * 7 + [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
     "vatss_tc_attention": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p] + [ctypes.c_int] * 7 + [ctypes.c_void_p]),
-    "vatss_tc_tail": (ctypes.c_int, [ctypes.POINTER(ModelDesc), ctypes.POINTER(ctypes.c_void_p), ctypes.c_int,
+    "vatss_generic_gemm": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_longlong] + [ctypes.c_void_p] * 4 +
+                           [ctypes.c_longlong, ctypes.c_void_p, ctypes.c_longlong, ctypes.c_longlong, ctypes.c_int,
+                            ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]),
+    "vatss_generic_layernorm": (ctypes.c_int, [ctypes.c_void_p] * 5 + [ctypes.c_longlong, ctypes.c_int, ctypes.c_int,
+                                                                       ctypes.c_void_p]),
+    "vatss_generic_attention": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p] + [ctypes.c_int] * 6 +
+                                [ctypes.c_void_p]),
+    "vatss_generic_lstm": (ctypes.c_int, [ctypes.c_void_p] * 4 + [ctypes.c_int] * 6 + [ctypes.c_void_p]),
+    "vatss_tc_tail": (ctypes.c_int,[ctypes.POINTER(ModelDesc), ctypes.POINTER(ctypes.c_void_p), ctypes.c_int,
                                      ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int,
                                      ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t,
                                      ctypes.c_void_p]),

@@ -427,6 +427,37 @@ int vatss_tc_attention(const void* qkv16, void* out16, int mode, int B, int S, i
                               (cudaStream_t)stream);
 }
 
+int vatss_generic_gemm(const float* A, long long lda, const float* W, const float* bias, const float* bias2,
+                       const float* R, long long ldr, float* out, long long ldc, long long M, int NOUT, int K, int act,
+                       const float* prelu_a, void* stream) {
+  VATSS_CHECK_ARG(A && W && out && M >= 0 && NOUT > 0 && K > 0, "generic_gemm: bad argument");
+  VATSS_CHECK_ARG(act >= 0 && act <= 2 && (act != 2 || prelu_a), "generic_gemm: act %d needs its PReLU slope", act);
+  return launch_gemm_simt(A, lda, W, bias, bias2, R, ldr, out, ldc, M, NOUT, K, act, prelu_a, (cudaStream_t)stream);
+}
+
+int vatss_generic_layernorm(const float* in, const float* res, const float* w, const float* b, float* out,
+                            long long rows, int N, int mode, void* stream) {
+  VATSS_CHECK_ARG(in && w && b && out && rows >= 0 && N > 0 && (mode == 0 || mode == 1),
+                  "generic_layernorm: bad argument");
+  return launch_layernorm(in, res, w, b, out, rows, N, mode, (cudaStream_t)stream);
+}
+
+int vatss_generic_attention(const float* qkv, float* out, int mode, int B, int S, int C, int N, int heads,
+                            void* stream) {
+  VATSS_CHECK_ARG(qkv && out && (mode == 0 || mode == 1) && B > 0 && S > 0 && C > 0 && N > 0,
+                  "generic_attention: bad argument");
+  const SeqMap map = mode == 0 ? intra_map(B, S, C) : inter_map(B, S, C);
+  return launch_attention_simt(qkv, out, map, N, heads, (cudaStream_t)stream);
+}
+
+int vatss_generic_lstm(const float* pre, const float* whh_f, const float* whh_r, float* out, int mode, int B, int S,
+                       int C, int H, int ndir, void* stream) {
+  VATSS_CHECK_ARG(pre && whh_f && out && (ndir == 1 || (ndir == 2 && whh_r)), "generic_lstm: bad argument");
+  VATSS_CHECK_ARG((mode == 0 || mode == 1) && B > 0 && S > 0 && C > 0, "generic_lstm: bad shape");
+  const SeqMap map = mode == 0 ? intra_map(B, S, C) : inter_map(B, S, C);
+  return launch_lstm_simt(pre, whh_f, whh_r, out, map, H, ndir, (cudaStream_t)stream);
+}
+
 int vatss_tc_tail(const vatss_model_desc* d, const float* const* params, int n_params, const void* packed,
                   const void* x16, const float* enc, int B, int T, float* s1_pred, float* s2_pred, void* workspace,
                   size_t workspace_bytes, void* stream) {

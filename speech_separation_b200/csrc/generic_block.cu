@@ -1,4 +1,5 @@
-// GENERIC engine of the dual-path blocks: fp32 SIMT kernels that accept any model dimensions.
+// GENERIC engine of the dual-path blocks: fp32 SIMT kernels for N <= 256, H <= 128 (multiple of 4) and
+// head dim <= 64, at any sequence length (W_hh is held in fp16 for H >= 108, see launch_lstm_simt).
 // They carry the small / odd configurations (the tiny golden fixtures, audio-only N=64 models
 // until the tensor engine covers them) and are the on-device cross-check for the tcgen05
 // TENSOR engine (tc_*.cu).  Semantics follow src/model/dptn.py:36-52 (TransformerDPRNN) and
@@ -150,89 +151,109 @@ int launch_layernorm(const float* in, const float* res, const float* w, const fl
 // ----------------------------------------------------------------------------------------
 // Multi-head self-attention core: out[row, h*hd:(h+1)*hd] = softmax(q k^T / sqrt(hd)) v
 // qkv rows are (q | k | v), each N wide (nn.MultiheadAttention packed in_proj, dptn.py:16-21).
-// One CTA per (sequence, head); K and V of the head staged in shared memory; one query per
-// thread with an online softmax.
+// One CTA per (sequence, head, block of 128 queries); one query per thread with an online
+// softmax.  K and V of the head stream through shared memory in tiles of ATT_TILE_FLOATS / HDMAX
+// keys, so any sequence length runs.  HDMAX is the register size of q and the accumulator: EXACT
+// instances (hd = HDMAX, the powers of two) run unpredicated loops, the others take any runtime
+// hd <= HDMAX (so every hd up to 64 runs).
 // ----------------------------------------------------------------------------------------
-template <int HD>
-__global__ void __launch_bounds__(128)
-k_attention_simt(const float* __restrict__ qkv, float* __restrict__ out, SeqMap map, int N) {
-  extern __shared__ float smem[];
+constexpr int ATT_THREADS = 128;
+constexpr int ATT_TILE_FLOATS = 4096;  // per operand: 16 KB of K and 16 KB of V
+
+template <int HDMAX, bool EXACT>
+__global__ void __launch_bounds__(ATT_THREADS)
+k_attention_simt(const float* __restrict__ qkv, float* __restrict__ out, SeqMap map, int N, int hd_rt) {
+  const int hd = EXACT ? HDMAX : hd_rt;
+  constexpr int TILE = ATT_TILE_FLOATS / HDMAX;  // keys per tile
+  __shared__ float sK[TILE * HDMAX];             // [TILE][HDMAX], columns >= hd unused
+  __shared__ float sV[TILE * HDMAX];
   const int g = blockIdx.x, h = blockIdx.y;
   const int len = map.len;
-  float* sK = smem;             // [len][HD]
-  float* sV = smem + len * HD;  // [len][HD]
-  for (int i = threadIdx.x; i < len * HD; i += blockDim.x) {
-    const int t = i / HD, d = i - t * HD;
-    const long long r = map.row(g, t);
-    sK[i] = qkv[r * 3 * N + N + h * HD + d];
-    sV[i] = qkv[r * 3 * N + 2 * N + h * HD + d];
-  }
-  __syncthreads();
-  const float scale = rsqrtf((float)HD);
-  for (int t = threadIdx.x; t < len; t += blockDim.x) {
-    const long long r = map.row(g, t);
-    float q[HD], acc[HD];
+  const int t = blockIdx.z * ATT_THREADS + threadIdx.x;
+  const bool active = t < len;
+  const long long r = active ? map.row(g, t) : 0;
+  const float scale = rsqrtf((float)hd);
+  float q[HDMAX], acc[HDMAX];
 #pragma unroll
-    for (int d = 0; d < HD; ++d) {
-      q[d] = qkv[r * 3 * N + h * HD + d] * scale;
-      acc[d] = 0.f;
+  for (int d = 0; d < HDMAX; ++d) {
+    q[d] = (active && (EXACT || d < hd)) ? qkv[r * 3 * N + h * hd + d] * scale : 0.f;
+    acc[d] = 0.f;
+  }
+  float m = -INFINITY, l = 0.f;
+  for (int j0 = 0; j0 < len; j0 += TILE) {
+    const int nk = min(TILE, len - j0);
+    __syncthreads();  // the previous tile has been consumed
+    for (int i = threadIdx.x; i < nk * hd; i += ATT_THREADS) {
+      const int j = i / hd, d = i - j * hd;
+      const long long rk = map.row(g, j0 + j);
+      sK[j * HDMAX + d] = qkv[rk * 3 * N + N + h * hd + d];
+      sV[j * HDMAX + d] = qkv[rk * 3 * N + 2 * N + h * hd + d];
     }
-    float m = -INFINITY, l = 0.f;
-    for (int j = 0; j < len; ++j) {
+    __syncthreads();
+    if (!active) continue;
+    for (int j = 0; j < nk; ++j) {
       float s = 0.f;
 #pragma unroll
-      for (int d = 0; d < HD; ++d) s = fmaf(q[d], sK[j * HD + d], s);
+      for (int d = 0; d < HDMAX; ++d)
+        if (EXACT || d < hd) s = fmaf(q[d], sK[j * HDMAX + d], s);
       if (s > m) {
         const float c = expf(m - s);
         l *= c;
 #pragma unroll
-        for (int d = 0; d < HD; ++d) acc[d] *= c;
+        for (int d = 0; d < HDMAX; ++d) acc[d] *= c;
         m = s;
       }
       const float p = expf(s - m);
       l += p;
 #pragma unroll
-      for (int d = 0; d < HD; ++d) acc[d] = fmaf(p, sV[j * HD + d], acc[d]);
+      for (int d = 0; d < HDMAX; ++d)
+        if (EXACT || d < hd) acc[d] = fmaf(p, sV[j * HDMAX + d], acc[d]);
     }
-    const float inv = 1.f / l;
-#pragma unroll
-    for (int d = 0; d < HD; ++d) out[r * N + h * HD + d] = acc[d] * inv;
   }
+  if (!active) return;
+  const float inv = 1.f / l;
+#pragma unroll
+  for (int d = 0; d < HDMAX; ++d)
+    if (EXACT || d < hd) out[r * N + h * hd + d] = acc[d] * inv;
 }
 
-template <int HD>
+template <int HDMAX, bool EXACT>
 static int attention_launch(const float* qkv, float* out, SeqMap map, int N, int heads, cudaStream_t st) {
-  const size_t smem = (size_t)2 * map.len * HD * sizeof(float);
-  VATSS_CHECK_ARG(smem <= 200 * 1024, "attention: sequence length %d too long for the generic kernel", map.len);
-  VATSS_CUDA_OK(cudaFuncSetAttribute(k_attention_simt<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)smem));
-  dim3 grid(map.G, heads);
-  k_attention_simt<HD><<<grid, 128, smem, st>>>(qkv, out, map, N);
+  VATSS_CHECK_ARG(heads <= 65535 && ceil_div(map.len, ATT_THREADS) <= 65535,
+                  "attention: %d heads x length %d exceed the grid", heads, map.len);
+  dim3 grid(map.G, heads, ceil_div(map.len, ATT_THREADS));
+  k_attention_simt<HDMAX, EXACT><<<grid, ATT_THREADS, 0, st>>>(qkv, out, map, N, N / heads);
   VATSS_LAUNCH_OK();
   return 0;
 }
 
 int launch_attention_simt(const float* qkv, float* out, SeqMap map, int N, int heads, cudaStream_t st) {
   VATSS_CHECK_ARG(heads > 0 && N % heads == 0, "attention: N=%d not divisible by heads=%d", N, heads);
-  if (map.G == 0) return 0;
-  switch (N / heads) {
-    case 1: return attention_launch<1>(qkv, out, map, N, heads, st);
-    case 2: return attention_launch<2>(qkv, out, map, N, heads, st);
-    case 4: return attention_launch<4>(qkv, out, map, N, heads, st);
-    case 8: return attention_launch<8>(qkv, out, map, N, heads, st);
-    case 16: return attention_launch<16>(qkv, out, map, N, heads, st);
-    case 32: return attention_launch<32>(qkv, out, map, N, heads, st);
-    case 64: return attention_launch<64>(qkv, out, map, N, heads, st);
-    default: set_error("attention: head dim %d unsupported", N / heads); return -1;
+  const int hd = N / heads;
+  VATSS_CHECK_ARG(hd <= 64, "attention: head dim %d unsupported by the generic kernel (max 64)", hd);
+  if (map.G == 0 || map.len == 0) return 0;
+  switch (hd) {
+    case 1: return attention_launch<1, true>(qkv, out, map, N, heads, st);
+    case 2: return attention_launch<2, true>(qkv, out, map, N, heads, st);
+    case 4: return attention_launch<4, true>(qkv, out, map, N, heads, st);
+    case 8: return attention_launch<8, true>(qkv, out, map, N, heads, st);
+    case 16: return attention_launch<16, true>(qkv, out, map, N, heads, st);
+    case 32: return attention_launch<32, true>(qkv, out, map, N, heads, st);
+    case 64: return attention_launch<64, true>(qkv, out, map, N, heads, st);
+    default: break;
   }
+  if (hd < 8) return attention_launch<8, false>(qkv, out, map, N, heads, st);
+  if (hd < 16) return attention_launch<16, false>(qkv, out, map, N, heads, st);
+  if (hd < 32) return attention_launch<32, false>(qkv, out, map, N, heads, st);
+  return attention_launch<64, false>(qkv, out, map, N, heads, st);
 }
 
 // ----------------------------------------------------------------------------------------
 // LSTM recurrence (one layer, h0=c0=0, gate order i,f,g,o): nn.LSTM, dptn.py:23-29,49.
 //   gates_t = pre[row(g,t)] + h_{t-1} Whh^T ; c = sig(f) c + sig(i) tanh(g) ; h = sig(o) tanh(c)
 // `pre` already holds x W_ih^T + b_ih + b_hh.  One CTA owns LSTM_ST sequences of one
-// direction for all time steps; Whh^T lives in shared memory for the whole kernel (fp32 when it
-// fits, fp16 otherwise); thread j owns gate column j.
+// direction for all time steps; Whh^T lives in shared memory for the whole kernel (fp32 for
+// H <= 104, fp16 for H >= 108); thread j owns gate column j.
 // ----------------------------------------------------------------------------------------
 constexpr int LSTM_ST = 8;
 
@@ -321,6 +342,8 @@ int launch_lstm_simt(const float* pre, const float* Whh_f, const float* Whh_r, f
   const size_t state = (size_t)(2 * LSTM_ST * H + LSTM_ST * 4 * H) * sizeof(float);
   const size_t w32 = (size_t)4 * H * H * sizeof(float);
   dim3 grid(ceil_div(map.G, LSTM_ST), ndir);
+  // fp32 except W_hh in fp16 for H >= 108: W_hh^T stays fp32 in shared memory while 16H^2 + 192H <= 200 KB
+  // (H <= 104); above that it is rounded to fp16 (relative error 2^-11 per weight), the rest stays fp32.
   if (state + w32 <= 200 * 1024) {
     VATSS_CUDA_OK(cudaFuncSetAttribute(k_lstm_simt<float>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)(state + w32)));
