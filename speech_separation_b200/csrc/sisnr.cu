@@ -72,6 +72,11 @@ __device__ __forceinline__ PairMoments centred(const double* m, int ip, int ig, 
   return r;
 }
 
+// Residual power ||p_c - a g_c||^2 = pp - dot^2/gg of the eps-free loss, shared by the forward and the backward so that
+// both see the same value.  For a near-exact estimate the cancellation of the raw-moment centring can make it zero or
+// negative: the forward then reports -inf and the backward writes a zero gradient for that prediction.
+__device__ __forceinline__ double loss_residual(const PairMoments& pm) { return pm.pp - pm.dot * pm.dot / pm.gg; }
+
 __global__ void __launch_bounds__(256)
 k_sisnr_finalize(const double* __restrict__ scratch, int B, int T, int chunks, int has_mix,
                  double* __restrict__ rows, double* __restrict__ rows_loss, double* __restrict__ summary) {
@@ -101,8 +106,8 @@ k_sisnr_finalize(const double* __restrict__ scratch, int B, int T, int chunks, i
       if (q < 4) {
         // reference loss form, no eps: signal = dot^2/gg, noise = pp - dot^2/gg
         const double s = pm.dot * pm.dot / pm.gg;
-        double n = pm.pp - s;
-        if (n < 0.0) n = 0.0;   // perfect estimate: rounding may push the residual power below zero
+        double n = loss_residual(pm);
+        if (n < 0.0) n = 0.0;   // perfect estimate: rounding may push the residual power below zero (-inf)
         rows_loss[b * 4 + q] = -20.0 * log10(s / n);
       }
     }
@@ -134,6 +139,7 @@ int launch_pit_sisnr(const float* s1p, const float* s2p, const float* s1, const 
                      int B, int T, double* rows, double* rows_loss, double* summary, double* scratch,
                      cudaStream_t st) {
   VATSS_CHECK_ARG(B > 0 && T > 0, "pit_sisnr: empty batch (B=%d, T=%d)", B, T);
+  VATSS_CHECK_ARG(B <= 65535, "pit_sisnr: batch of %d utterances (at most 65535)", B);
   const int chunks = sisnr_chunks(T);
   dim3 grid(chunks, B);
   k_sisnr_moments<<<grid, 256, 0, st>>>(s1p, s2p, s1, s2, mix, T, chunks, scratch);
@@ -204,6 +210,7 @@ int launch_pit_sisdr(const float* s1p, const float* s2p, const float* s1, const 
 //   d l / d p = -(40 / ln 10) ( g_c / <g_c, p_c>  -  e / ||e||^2 )        (g_c and e are zero-mean: the centring Jacobian is I)
 // pi is the permutation the forward chose for the WHOLE batch (summary[1], summary[2]); the per-row centred moments come
 // from the forward's scratch (raw chunk sums), so the backward reads the four waveforms once and writes two gradients.
+// A prediction whose residual power (loss_residual) is <= 0, where the forward reports -inf, gets a zero gradient.
 // ------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
 k_sisnr_loss_backward(const float* __restrict__ s1p, const float* __restrict__ s2p, const float* __restrict__ s1,
@@ -226,15 +233,16 @@ k_sisnr_loss_backward(const float* __restrict__ s1p, const float* __restrict__ s
   const PairMoments c = centred(m, 1, swap ? 2 : 3, swap ? 13 : 11, invT);
   const double mp1 = m[0] * invT, mp2 = m[1] * invT, mg1 = m[swap ? 3 : 2] * invT, mg2 = m[swap ? 2 : 3] * invT;
   const double al1 = a.dot / a.gg, al2 = c.dot / c.gg;
-  const double n1 = a.pp - a.dot * a.dot / a.gg, n2 = c.pp - c.dot * c.dot / c.gg;
+  const double n1 = loss_residual(a), n2 = loss_residual(c);
+  // the forward clamped a residual <= 0 and reported -inf: no descent direction, a zero gradient (NaN stays NaN)
   const float* t1 = swap ? s2 : s1;
   const float* t2 = swap ? s1 : s2;
   const size_t base = (size_t)b * T;
   for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < T; t += gridDim.x * blockDim.x) {
     const double gc1 = (double)t1[base + t] - mg1, gc2 = (double)t2[base + t] - mg2;
     const double e1 = (double)s1p[base + t] - mp1 - al1 * gc1, e2 = (double)s2p[base + t] - mp2 - al2 * gc2;
-    g1[base + t] = (float)(up * (gc1 / a.dot - e1 / n1));
-    g2[base + t] = (float)(up * (gc2 / c.dot - e2 / n2));
+    g1[base + t] = n1 <= 0.0 ? 0.0f : (float)(up * (gc1 / a.dot - e1 / n1));
+    g2[base + t] = n2 <= 0.0 ? 0.0f : (float)(up * (gc2 / c.dot - e2 / n2));
   }
 }
 
@@ -242,6 +250,7 @@ int launch_pit_sisnr_backward(const float* s1p, const float* s2p, const float* s
                               const double* scratch, const double* summary, const float* grad_out, float* g1, float* g2,
                               cudaStream_t st) {
   VATSS_CHECK_ARG(B > 0 && T > 0, "pit_sisnr_backward: empty batch (B=%d, T=%d)", B, T);
+  VATSS_CHECK_ARG(B <= 65535, "pit_sisnr_backward: batch of %d utterances (at most 65535)", B);
   const int chunks = sisnr_chunks(T);
   int gx = (T + 256 * 8 - 1) / (256 * 8);
   if (gx < 1) gx = 1;

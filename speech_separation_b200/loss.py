@@ -9,12 +9,33 @@ Python `if loss_perm_2 < loss_perm_1` there is no host synchronisation.
 The loss is differentiable with respect to the predictions: when `s1_pred` / `s2_pred` require grad, `SiSNRWavLoss`
 returns a tensor whose `.backward()` (src/trainer/trainer.py:46) runs `vatss_pit_sisnr_backward` - one more pass over the
 four waveforms, reusing the forward's moments and its batch-level permutation.  (The separation models themselves are
-forward-only; this is the first piece of SURVEY.md §8f rank 2.)
+forward-only; this is the first piece of SURVEY.md §8f rank 2.)  `SiSNRLoss` is differentiable the same way.
+
+The moments are raw fp64 sums, centred algebraically, so for a near-exact estimate the residual power pp - dot^2/gg can
+round to zero or below.  The forward then reports -inf for that pair (the loss has no finite minimum there) and the
+backward returns a zero gradient for that prediction: -inf offers no descent direction.  A silent target gives NaN in
+both.
 """
+import math
+
 import torch
 from torch import nn
 
 from . import _lib
+
+
+MAX_B = 65535   # utterances per call: the kernels put the batch in grid.y
+
+
+def _batch_dims(shape):
+    """(B, T) of a (..., T) batch; raises ValueError for an empty or too large batch, before any device work."""
+    T = shape[-1] if len(shape) else 0
+    B = math.prod(shape[:-1]) if T > 0 else 0
+    if B == 0 or T == 0:
+        raise ValueError("empty batch")
+    if B > MAX_B:
+        raise ValueError(f"batch of {B} utterances: at most {MAX_B}")
+    return B, T
 
 
 def pit_sisnr_all(s1_pred, s2_pred, s1, s2, mix=None):
@@ -24,20 +45,17 @@ def pit_sisnr_all(s1_pred, s2_pred, s1, s2, mix=None):
     rows_loss: per-utterance reference-loss values of the first four pairs;
     summary: [loss, loss_perm1, loss_perm2, SI-SNR(PIT), SI-SNRi, mean SI-SNR(mix,s1), mean SI-SNR(mix,s2), B].
     """
+    shape = s1_pred.shape
+    for name, t in (("s2_pred", s2_pred), ("s1", s1), ("s2", s2), ("mix", mix)):
+        if t is not None and t.shape != shape:
+            raise ValueError(f"{name} has shape {tuple(t.shape)}, expected {tuple(shape)}")
+    B, T = _batch_dims(shape)
     s1_pred = _lib.f32c(s1_pred, "s1_pred")
     s2_pred = _lib.f32c(s2_pred, "s2_pred")
     s1 = _lib.f32c(s1, "s1")
     s2 = _lib.f32c(s2, "s2")
     if mix is not None:
         mix = _lib.f32c(mix, "mix")
-    shape = s1_pred.shape
-    for name, t in (("s2_pred", s2_pred), ("s1", s1), ("s2", s2), ("mix", mix)):
-        if t is not None and t.shape != shape:
-            raise ValueError(f"{name} has shape {tuple(t.shape)}, expected {tuple(shape)}")
-    T = shape[-1]
-    B = s1_pred.numel() // T if T > 0 else 0
-    if B == 0 or T == 0:
-        raise ValueError("empty batch")
     lib = _lib.load()
     dev = s1_pred.device
     chunks = lib.vatss_sisnr_chunks(T)
@@ -58,10 +76,9 @@ class _PitSisnrLoss(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, s1_pred, s2_pred, s1, s2):
+        B, T = _batch_dims(s1_pred.shape)
         s1_pred, s2_pred, s1, s2 = (_lib.f32c(t.detach(), n) for t, n in
                                     ((s1_pred, "s1_pred"), (s2_pred, "s2_pred"), (s1, "s1"), (s2, "s2")))
-        T = s1_pred.shape[-1]
-        B = s1_pred.numel() // T
         lib = _lib.load()
         dev = s1_pred.device
         chunks = lib.vatss_sisnr_chunks(T)
@@ -92,9 +109,16 @@ class _PitSisnrLoss(torch.autograd.Function):
 
 
 class SiSNRLoss(nn.Module):
-    """Single-pair loss: mean_b[-20 log10(||a g||^2 / ||p - a g||^2)] (ss_losses.py:100-114)."""
+    """Single-pair loss: mean_b[-20 log10(||a g||^2 / ||p - a g||^2)] (ss_losses.py:100-114).
+
+    Differentiable with respect to `pred`: the pair is passed as both PIT pairs, whose moments are then bitwise equal, so
+    the kernel keeps permutation 1 and the value is the single-pair mean; the two 1/(2B) gradient halves add up to 1/B."""
 
     def forward(self, pred, gt, **batch):
+        if torch.is_grad_enabled() and pred.requires_grad:
+            if gt.shape != pred.shape:
+                raise ValueError(f"gt has shape {tuple(gt.shape)}, expected {tuple(pred.shape)}")
+            return _PitSisnrLoss.apply(pred, pred, gt, gt)
         _, rows_loss, _ = pit_sisnr_all(pred, pred, gt, gt)
         return rows_loss[:, 0].mean().float()
 
